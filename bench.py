@@ -2,7 +2,7 @@
 """bench.py -- the hot-path benchmark (BASELINE.json metric: units/s on synthetic
 4096x3000 mold images with the reference's grid.json grid).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one pass of the full per-unit inspection path (segmentation +
 defect pass + verdict) over one batch of `--images` (default 64 = configs[1])
@@ -12,6 +12,9 @@ masks + records out, copies inside the timed region).  Multi-GPU (torchrun, one
 process per GPU): configs[2], 1024 frames sharded by image; the per-unit record
 table is gathered by the kernel itself over NVLink peer memory and verified on
 rank 0 against an NCCL all-gather and a 1-rank run.
+
+`--dump-outputs DIR` writes what the last timed step computed (see `dump_outputs`) as DIR/<name>.npy, so that two
+builds of the project can be compared output for output on the same inputs.
 
 `--impl reference` times the reference's own CPU path (the cv2 oracle port,
 oracle/ref_cv2.py -- the reference itself needs PyQt6 and is absent on the GPU
@@ -89,6 +92,32 @@ def make_frames(seeds):
     from vi_b200 import synth
     boxes = [b for b, _ in grid_boxes()]
     return [synth.make_frame(s, boxes, H=H, W=W) for s in seeds]
+
+
+# --------------------------------------------------------------------------- output dump
+DUMP_MASK_UNITS = 48                       # units whose masks are dumped: both full mask sets are 612 MB at configs[1]
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, insp, rec, d_seg, d_def):
+    """Writes the outputs of one batch call as float arrays: every record field as record_<field>.npy [images, units]
+    (float64: the int32 fields and the float64 centroids are exact), and the seg / defect masks (0 or 255) of a fixed,
+    seeded sample of the batch's units as seg_masks.npy / defect_masks.npy [k, h, w] float32, with the sampled
+    (image, unit) pairs in sample_units.npy [k, 2]."""
+    n_units = insp.n_units
+    rec = rec.reshape(-1, n_units)
+    arrays = {f"record_{k}": rec[k].astype(np.float64) for k in rec.dtype.names}
+    n_all = rec.size
+    pick = np.sort(np.random.default_rng(0).choice(n_all, size=min(DUMP_MASK_UNITS, n_all), replace=False))
+    arrays["sample_units"] = np.stack([pick // n_units, pick % n_units], axis=1).astype(np.float64)
+    for name, flat in (("seg_masks", d_seg), ("defect_masks", d_def)):
+        arrays[name] = np.stack([insp.split_masks(flat, int(p // n_units))[int(p % n_units)].cpu().numpy()
+                                 for p in pick]).astype(np.float32)
+    total = sum(a.nbytes for a in arrays.values())
+    assert total <= DUMP_MAX_BYTES, f"output dump of {total} bytes exceeds {DUMP_MAX_BYTES}"
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 # --------------------------------------------------------------------------- clocks
@@ -273,6 +302,8 @@ def run_gpu_arm(args, rank, world, local_rank):
     value = units_per_step / (ms_per_step * 1e-3)
 
     rec = d_rec.cpu().numpy().view(vi_b200.RECORD_DTYPE).reshape(-1)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, insp, rec, d_seg, d_def)
     ng_gpu = int((rec['status'] == vi_b200.STATUS_NG).sum())
     table_check = None
     if world > 1:
@@ -428,7 +459,13 @@ def main():
     ap.add_argument("--no-ingest", action="store_true", help="skip the frame-ingest streaming kernels")
     ap.add_argument("--cpu-passes", type=int, default=40, help="passes over the sample frames in the cpu_baseline leg (~10 s)")
     ap.add_argument("--ref-passes", type=int, default=8, help="passes over the sample frames per step of the reference arm")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's records and a seeded sample of its masks as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the CUDA path's outputs; the reference arm keeps only NG counts")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
