@@ -130,11 +130,10 @@ int vi_inspect_batch(vi_ctx* ctx, const uint8_t* d_frames, int n_images, int W, 
 int vi_set_seg_stats_output(vi_ctx* ctx, int64_t* d_stats);
 
 /* Same, from and to HOST buffers: works through the batch in chunks on internal
- * streams so that upload, compute and download overlap; blocks until done.  With
- * VI_HOST_UPLOAD=mapped in the environment, pinned frames (cudaHostAlloc /
- * cudaHostRegister, e.g. torch pin_memory) are not copied: the kernel gathers the
- * unit crops from them in place over the host link.  h_seg_masks / h_defect_masks may be NULL to skip
- * that download.  This is the end-to-end call bench.py times as `e2e`. */
+ * streams so that upload, compute and download overlap; blocks until done.  Pinned
+ * and pageable frames take the same path: the frame rows that some unit covers are
+ * copied to a device staging buffer.  h_seg_masks / h_defect_masks may be NULL to
+ * skip that download.  This is the end-to-end call bench.py times as `e2e`. */
 int vi_inspect_batch_host(vi_ctx* ctx, const uint8_t* h_frames, int n_images, int W, int H,
                           int64_t row_pitch, int64_t image_stride, const vi_params* params,
                           uint8_t* h_seg_masks, uint8_t* h_defect_masks, vi_unit_record* h_records);
@@ -174,9 +173,8 @@ int vi_peer_table_destroy(vi_ctx* ctx, void* d_table);
 int vi_peer_table_read(vi_ctx* ctx, const void* d_table, int64_t n_records, vi_unit_record* h_out);   /* blocking download */
 int vi_set_record_peers(vi_ctx* ctx, void* const* d_tables, int n, int image_mul, int image_add);
 
-/* Bytes vi_inspect_batch_host moves host -> device for n_images frames.  Pageable frames: only the frame rows that
- * some unit covers are copied (one strided copy per merged row interval) -- pass their row_pitch.  With
- * VI_HOST_UPLOAD=mapped, pinned frames are read in place by the crop gather, unit pixels only -- pass row_pitch = 0. */
+/* Bytes vi_inspect_batch_host moves host -> device for n_images frames of the given row_pitch: only the frame rows
+ * that some unit covers are copied (one strided copy per merged row interval).  0 when row_pitch <= 0. */
 int64_t vi_host_upload_bytes(vi_ctx* ctx, int n_images, int64_t row_pitch);
 
 /* ---- frame ingest (device pointers, asynchronous on `stream`) ---------------- */

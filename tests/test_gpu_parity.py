@@ -381,8 +381,8 @@ def _records_equal(a, b):
 @pytest.mark.parametrize("pinned", [False, True])
 def test_host_batch_multi_chunk(insp, golden, monkeypatch, chunk, pinned):
     """The chunked pipeline of the host-buffer call: slot wrap-around (5 images, 1 or 2 per chunk, 3 slots), the
-    chunk-local -> batch-global image index, exclusions and centroid shifts, pinned (read in place by the crop gather)
-    and pageable (staged) frames -- every record field and both mask sets against the device-resident call."""
+    chunk-local -> batch-global image index, exclusions and centroid shifts, pinned and pageable frames -- every record
+    field and both mask sets against the device-resident call."""
     import torch
     g = golden('config4')
     meta = g.meta
@@ -398,7 +398,6 @@ def test_host_batch_multi_chunk(insp, golden, monkeypatch, chunk, pinned):
     assert (rec_d['dx'] != 0).any() or (rec_d['dy'] != 0).any()
     monkeypatch.setenv("VI_HOST_CHUNK", chunk)
     if pinned:
-        monkeypatch.setenv("VI_HOST_UPLOAD", "mapped")
         ht = torch.empty(frames.shape, dtype=torch.uint8, pin_memory=True)
         ht.numpy()[...] = frames
         hf = ht.numpy()
@@ -706,39 +705,38 @@ def test_ragged_grid_and_unaligned_frames(insp):
                     assert rec[fi, u][k] == o[k], (params, fi, u, k, rec[fi, u][k], o[k])
 
 
-def test_async_gather_variants_agree(insp, monkeypatch):
-    """The default kernel fetches the next unit's crop asynchronously, as tensor-map boxes (cp.async.bulk.tensor) or,
-    with VI_GATHER=rows, as one bulk copy per row; both undo the crop's byte phase (x0 & 15) afterwards.  Units at
-    every byte phase and of several sizes, on 16-byte aligned frames: both variants against the cv2 oracle."""
+def test_async_gather_variants_agree(insp):
+    """The default kernel fetches the next unit's crop asynchronously and undoes the crop's byte phase (x0 & 15)
+    afterwards: as tensor-map boxes (cp.async.bulk.tensor) when the box tiles of the grid's largest unit fit the staging
+    area (gray crop + first mask), else as one bulk copy per row.  Units at every byte phase, on 16-byte aligned frames,
+    against the cv2 oracle, one grid per variant:
+    boxes: units of several sizes up to 316 x 315 (3 frames: every unit is the first of its CTA, fetched as boxes);
+    rows:  16 units of 150 x 230 -- the boxes need 176 B x 232 rows = 40,832 B, more than the 40,496 B of gray + mask,
+           the row copies at most 176 x 230 = 40,480 B.  20 frames, so that every CTA (one per SM) fetches later units."""
     import torch
-    W, H = 1024, 420
-    boxes = [((3 + 37 * i + (i % 16), 8 + 5 * (i % 3), 36, 40), i) for i in range(16)]                   # x0 & 15 takes many values
-    boxes += [((16, 70, 316, 315), 16), ((349, 72, 316, 315), 17), ((680, 75, 300, 200), 18), ((683, 290, 97, 111), 19)]
-    frames = np.stack([synth.make_frame(s, [b for b, _ in boxes], H=H, W=W, inset=5, jitter=2) for s in (31, 32, 33)])
-    d = torch.from_numpy(frames).cuda()
-    outs = []
-    for mode in ("", "rows"):
-        if mode: monkeypatch.setenv("VI_GATHER", mode)
-        else: monkeypatch.delenv("VI_GATHER", raising=False)
+    boxes_grid = [((3 + 37 * i + (i % 16), 8 + 5 * (i % 3), 36, 40), i) for i in range(16)]          # x0 & 15 takes many values
+    boxes_grid += [((16, 70, 316, 315), 16), ((349, 72, 316, 315), 17), ((680, 75, 300, 200), 18), ((683, 290, 97, 111), 19)]
+    rows_grid = [((16 + 176 * j + 8 * r + j, 8 + 246 * r, 150, 230), 8 * r + j) for r in range(2) for j in range(8)]  # x0 & 15 = 0..15
+    for boxes, W, H, seeds in ((boxes_grid, 1024, 420, (31, 32, 33)), (rows_grid, 1424, 496, range(40, 60))):
+        frames = np.stack([synth.make_frame(s, [b for b, _ in boxes], H=H, W=W, inset=5, jitter=2) for s in seeds])
+        n = len(frames)
         insp.configure(Grid(boxes=boxes), is_reference=True)
-        rec, seg, dfm = insp.inspect_batch(d)
+        rec, seg, dfm = insp.inspect_batch(torch.from_numpy(frames).cuda())
         torch.cuda.synchronize()
-        outs.append((rec.cpu().numpy().view(vi_b200.RECORD_DTYPE).reshape(3, len(boxes)), seg.cpu().numpy().reshape(3, -1),
-                     dfm.cpu().numpy().reshape(3, -1)))
-    monkeypatch.delenv("VI_GATHER", raising=False)
-    assert np.array_equal(outs[0][1], outs[1][1]) and np.array_equal(outs[0][2], outs[1][2])
-    for k in ('otsu_t', 'seg_area', 'roi_area', 'defect_area', 'n_kept', 'status'):
-        assert np.array_equal(outs[0][0][k], outs[1][0][k]), k
-    rec, seg, dfm = outs[0]
-    for fi in range(3):
-        recs, osegs, odefs = R.inspect_frame(frames[fi], boxes, R.Params(), (), None, True)
-        segs = insp.split_masks(seg[fi]); defs = insp.split_masks(dfm[fi])
-        for u, o in enumerate(recs):
-            assert np.array_equal(segs[u], osegs[u]), (fi, u, 'seg')
-            ref = odefs[u] if odefs[u] is not None else np.zeros_like(defs[u])
-            assert np.array_equal(defs[u], ref), (fi, u, 'defect')
-            for k in ('seg_area', 'roi_area', 'defect_area', 'n_kept', 'status'):
-                assert rec[fi, u][k] == o[k], (fi, u, k)
+        rec = rec.cpu().numpy().view(vi_b200.RECORD_DTYPE).reshape(n, len(boxes))
+        seg = seg.cpu().numpy().reshape(n, -1); dfm = dfm.cpu().numpy().reshape(n, -1)
+        for fi in range(n):
+            recs, osegs, odefs = R.inspect_frame(frames[fi], boxes, R.Params(), (), None, True)
+            segs = insp.split_masks(seg[fi]); defs = insp.split_masks(dfm[fi])
+            for u, o in enumerate(recs):
+                (x, y, w, h), _ = boxes[u]
+                otsu = R.otsu_threshold(cv2.GaussianBlur(frames[fi, y:y + h, x:x + w], (3, 3), 0))
+                assert rec[fi, u]['otsu_t'] == otsu, (W, fi, u, 'otsu_t')
+                assert np.array_equal(segs[u], osegs[u]), (W, fi, u, 'seg')
+                ref = odefs[u] if odefs[u] is not None else np.zeros_like(defs[u])
+                assert np.array_equal(defs[u], ref), (W, fi, u, 'defect')
+                for k in ('seg_area', 'roi_area', 'defect_area', 'n_kept', 'status'):
+                    assert rec[fi, u][k] == o[k], (W, fi, u, k)
 
 
 def test_detect_defects_on_a_bright_region(insp):

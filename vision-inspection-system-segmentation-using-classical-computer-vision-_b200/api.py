@@ -177,8 +177,8 @@ class Inspector:
         return out
 
     def inspect_batch_host(self, frames: np.ndarray, params=None, want_masks=True, out=None, mask_format="bytes"):
-        """frames: host uint8 [n, H, W] (numpy; pinned memory -- e.g. a torch pin_memory tensor's .numpy() -- is read in
-        place by the device, pageable memory is staged).  mask_format: "bytes" (0/255, the reference's masks), "packed"
+        """frames: host uint8 [n, H, W] (numpy, pageable or pinned -- e.g. a torch pin_memory tensor's .numpy(); either
+        way the rows the grid covers are copied to the device).  mask_format: "bytes" (0/255, the reference's masks), "packed"
         (1 bit per pixel, see `unpack_masks`) or "none" (records only).
         Returns (records structured array, seg_masks u8 | None, defect_masks u8 | None)."""
         frames = _u8c(frames, "frames")

@@ -354,19 +354,22 @@ extern "C" int vi_set_seg_stats_output(vi_ctx* c, int64_t* d_stats) {
     return VI_OK;
 }
 
-extern "C" int64_t vi_host_upload_bytes(vi_ctx* c, int n_images, int64_t row_pitch) {
-    if (!c) return 0;
-    if (row_pitch <= 0) return (int64_t)c->grid.unit_px * n_images;          // mapped pinned frames: the crops only
-    std::vector<std::pair<int, int>> iv;
-    for (const int4& r : c->grid.rects) iv.emplace_back(r.y, r.y + r.w);
+// Merged [y0, y1) row intervals of the frame that some unit of the grid covers: the rows the host-buffer call uploads.
+static std::vector<std::pair<int, int>> covered_rows(const GridState& gs) {
+    std::vector<std::pair<int, int>> iv, rows;
+    for (const int4& r : gs.rects) iv.emplace_back(r.y, r.y + r.w);
     std::sort(iv.begin(), iv.end());
-    long long rows = 0;
-    int end = -1;
     for (const auto& p : iv) {
-        int a0 = std::max(p.first, end);
-        if (p.second > a0) rows += p.second - a0;
-        end = std::max(end, p.second);
+        if (!rows.empty() && p.first <= rows.back().second) rows.back().second = std::max(rows.back().second, p.second);
+        else rows.push_back(p);
     }
+    return rows;
+}
+
+extern "C" int64_t vi_host_upload_bytes(vi_ctx* c, int n_images, int64_t row_pitch) {
+    if (!c || row_pitch <= 0) return 0;
+    long long rows = 0;
+    for (const auto& iv : covered_rows(c->grid)) rows += iv.second - iv.first;
     return (int64_t)rows * row_pitch * n_images;
 }
 
@@ -600,7 +603,6 @@ static PFN_tmap_encode tmap_encoder() {
 
 static bool make_frame_tensor(KArgs& a, const GridState& gs) {
     a.tma_ok = 0;
-    if (const char* e = getenv("VI_GATHER")) { if (strcmp(e, "rows") == 0) return false; }      // VI_GATHER=rows: the per-row bulk copies
     PFN_tmap_encode enc = tmap_encoder();
     if (!enc) return false;
     // the aligned span of a crop: up to 15 bytes of phase in front; tiles of equal width (a multiple of 16) and whole
@@ -656,8 +658,6 @@ static int launch_units(vi_ctx* c, KArgs& a, const GridState& gs, cudaStream_t s
     a.arena_stride = astride;
     a.wmax = gs.wmax; a.hmax = gs.hmax;
     a.plan = gs.plan;
-    a.prof = (&gs == &c->grid) ? c->prof : nullptr;
-    if (&gs != &c->grid) a.seg_stats = nullptr;
     if (c->smem_set < gs.plan.total) {
         const int lim = c->smem_optin - c->smem_static;
         CU(cudaFuncSetAttribute(vi_unit_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
@@ -676,12 +676,11 @@ static int launch_units(vi_ctx* c, KArgs& a, const GridState& gs, cudaStream_t s
         CU(cudaGetLastError());
         return VI_OK;
     }
-    // The default configuration has its own instantiation (vi_unit.cuh: SPEC); VI_KERNEL=general switches it off.
+    // The default configuration has its own instantiation (vi_unit.cuh: SPEC).
     bool spec = a.mode == MODE_FULL && a.blur_k == 3 && a.se_k == 3 && a.p.seg_method == 0 && a.p.defect_method == 0 &&
                 !a.labels_out && !a.seg_stats && !a.seg_bits && !a.def_bits && !a.aux_mask && !a.stats_out &&
                 (a.row_pitch & 15) == 0 && (reinterpret_cast<uintptr_t>(a.frames) & 15) == 0 && (a.image_stride & 15) == 0 &&
                 rank_ws_bytes(gs.wmax, gs.hmax) + kOtsuWsBytes <= (long long)(kNumMasks - 1) * gs.plan.mask_bytes + gs.plan.ws_bytes && gs.plan.n_hist >= kWarps / 2;
-    if (spec) { const char* e = getenv("VI_KERNEL"); if (e && strcmp(e, "general") == 0) spec = false; }
     if (spec) make_frame_tensor(a, gs);
 #ifndef VI_CHECKED
     if (a.prof && spec) vi_unit_kernel<true, true, false><<<nblocks, kThreads, gs.plan.total, stream>>>(a);   // diagnostics build: phase timers
@@ -716,6 +715,18 @@ static void base_args(vi_ctx* c, KArgs& a, const GridState& gs) {
     a.image_mul = 1;
 }
 
+// What a batch over the user grid launches with besides its outputs: the frames, the context's tables (exclusions,
+// reference centroids) and its phase-profile buffer.
+static void batch_args(vi_ctx* c, KArgs& a, const uint8_t* frames, int n_images, int W, int H, int64_t row_pitch,
+                       int64_t image_stride) {
+    a.frames = frames; a.n_images = n_images; a.W = W; a.H = H; a.row_pitch = row_pitch; a.image_stride = image_stride;
+    a.excl = (const vi_excl*)c->d_excl.p; a.n_excl = (int)c->excl.size();
+    a.refc = c->has_refc ? (const double*)c->d_refc.p : nullptr;
+    a.is_reference = c->is_reference;
+    a.mode = MODE_FULL;
+    a.prof = c->prof;
+}
+
 extern "C" int vi_inspect_batch(vi_ctx* c, const uint8_t* d_frames, int n_images, int W, int H, int64_t row_pitch,
                                 int64_t image_stride, const vi_params* params, uint8_t* d_seg, uint8_t* d_def,
                                 int32_t* d_labels, vi_unit_record* d_rec, void* stream) {
@@ -729,12 +740,8 @@ extern "C" int vi_inspect_batch(vi_ctx* c, const uint8_t* d_frames, int n_images
     KArgs a;
     base_args(c, a, c->grid);
     if ((rc = fill_params(a, params))) return rc;
-    a.frames = d_frames; a.n_images = n_images; a.W = W; a.H = H; a.row_pitch = row_pitch; a.image_stride = image_stride;
-    a.excl = (const vi_excl*)c->d_excl.p; a.n_excl = (int)c->excl.size();
-    a.refc = c->has_refc ? (const double*)c->d_refc.p : nullptr;
-    a.is_reference = c->is_reference;
+    batch_args(c, a, d_frames, n_images, W, H, row_pitch, image_stride);
     a.seg_out = d_seg; a.def_out = d_def; a.labels_out = d_labels; a.rec = d_rec;
-    a.mode = MODE_FULL;
     a.seg_stats = c->seg_stats;
     a.seg_bits = c->seg_bits; a.def_bits = c->def_bits;
     a.n_peers = c->n_peers; a.image_mul = c->image_mul; a.image_base = c->image_add;
@@ -770,40 +777,16 @@ static int host_batch(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, i
     int chunk = std::max(1, (2 * c->sm_count + n_units - 1) / n_units);
     if (const char* e = getenv("VI_HOST_CHUNK")) { int v = atoi(e); if (v > 0) chunk = v; }
     chunk = std::min(chunk, n_images);
-    // Upload.  Default: one strided copy per merged row interval of the grid into a device staging buffer (the copy
-    // engine moves whole frame rows at the link rate).  VI_HOST_UPLOAD=mapped: pinned host frames that the device can
-    // address (cudaHostAlloc / cudaHostRegister under unified addressing) are not copied at all -- the crop gather of
-    // the kernel reads them in place over the host link, so only the pixels inside unit rects cross it (38.9 % of a
-    // frame for grid.json).  Measured on a B200 / PCIe Gen5 x16: the in-place gather is latency-bound per unit
-    // (16.2 ms per 64-frame step against 14.6 ms staged), so it is opt-in: it pays where the host link is shared.
-    const uint8_t* d_mapped = nullptr;
-    {
-        const char* e = getenv("VI_HOST_UPLOAD");
-        if (e && strcmp(e, "mapped") == 0) {
-            cudaPointerAttributes pa;
-            if (cudaPointerGetAttributes(&pa, h_frames) == cudaSuccess && pa.type == cudaMemoryTypeHost && pa.devicePointer)
-                d_mapped = (const uint8_t*)pa.devicePointer;
-            cudaGetLastError();                                       // an unregistered pointer may leave an error behind
-        }
-    }
     const size_t frame_bytes = (size_t)image_stride;
     for (int b = 0; b < kHostSlots; ++b) {
-        if (!d_mapped && (rc = c->hb_frames[b].ensure(frame_bytes * chunk))) return rc;
+        if ((rc = c->hb_frames[b].ensure(frame_bytes * chunk))) return rc;
         if (h_seg && (rc = c->hb_seg[b].ensure((size_t)ubytes * chunk))) return rc;
         if (h_def && (rc = c->hb_def[b].ensure((size_t)ubytes * chunk))) return rc;
         if ((rc = c->hb_rec[b].ensure(sizeof(vi_unit_record) * (size_t)n_units * chunk))) return rc;
     }
-    // merged [y0, y1) row intervals covered by the grid
-    std::vector<std::pair<int, int>> rows;
-    if (!d_mapped) {
-        std::vector<std::pair<int, int>> iv;
-        for (const int4& r : c->grid.rects) iv.emplace_back(r.y, r.y + r.w);
-        std::sort(iv.begin(), iv.end());
-        for (const auto& p : iv) {
-            if (!rows.empty() && p.first <= rows.back().second) rows.back().second = std::max(rows.back().second, p.second);
-            else rows.push_back(p);
-        }
-    }
+    // Upload: one strided copy per covered row interval into the slot's staging buffer (the copy engine moves whole
+    // frame rows at the link rate).
+    const std::vector<std::pair<int, int>> rows = covered_rows(c->grid);
     auto run_chunks = [&]() -> int {
         int slot = 0;
         for (int i0 = 0; i0 < n_images; i0 += chunk, slot = (slot + 1) % kHostSlots) {
@@ -816,19 +799,14 @@ static int host_batch(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, i
                                      (size_t)image_stride, bytes, n, cudaMemcpyHostToDevice, st));
             }
             KArgs a = a0;
-            a.frames = d_mapped ? d_mapped + (size_t)i0 * image_stride : (const uint8_t*)c->hb_frames[slot].p;
-            a.n_images = n; a.W = W; a.H = H; a.row_pitch = row_pitch; a.image_stride = image_stride;
+            batch_args(c, a, (const uint8_t*)c->hb_frames[slot].p, n, W, H, row_pitch, image_stride);
             a.image_base = i0;
-            a.excl = (const vi_excl*)c->d_excl.p; a.n_excl = (int)c->excl.size();
-            a.refc = c->has_refc ? (const double*)c->d_refc.p : nullptr;
-            a.is_reference = c->is_reference;
             if (mask_format == VI_MASKS_BYTES) {
                 a.seg_out = h_seg ? (uint8_t*)c->hb_seg[slot].p : nullptr; a.def_out = h_def ? (uint8_t*)c->hb_def[slot].p : nullptr;
             } else if (mask_format == VI_MASKS_PACKED) {
                 a.seg_bits = h_seg ? (uint32_t*)c->hb_seg[slot].p : nullptr; a.def_bits = h_def ? (uint32_t*)c->hb_def[slot].p : nullptr;
             }
             a.rec = (vi_unit_record*)c->hb_rec[slot].p;
-            a.mode = MODE_FULL;
             int r2;
             if ((r2 = launch_units(c, a, c->grid, st, slot))) return r2;
             if (h_seg) CU(cudaMemcpyAsync((uint8_t*)h_seg + (size_t)i0 * ubytes, c->hb_seg[slot].p, (size_t)ubytes * n, cudaMemcpyDeviceToHost, st));

@@ -43,7 +43,6 @@ constexpr int kWarps = kThreads / 32;
 constexpr int kOtsuWarp = kWarps - 1;   // this warp advances the exact Otsu recurrence while others walk columns (vi_rank.cuh)
 constexpr int kHistWords = 2048;   // per-warp lane-private histogram: [64 bin-quads][32 lanes] u32, 4 x 8-bit counters
 constexpr int kHistBytes = kHistWords * 4;
-constexpr int kMaxExcl = 32;
 constexpr int kMaxPeers = 8;       // GPUs of one NVSwitch domain that exchange record tables
 constexpr int kMaxTaps = 33;
 constexpr int kMaxSE = 33;
