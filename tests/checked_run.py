@@ -17,6 +17,7 @@ import vi_b200  # noqa: E402
 from vi_b200 import _lib, synth  # noqa: E402
 from vi_b200.grid import Grid  # noqa: E402
 from test_gpu_parity import adversarial_masks  # noqa: E402
+from test_gpu_unit_sequences import ARENA_UNITS, EXCL, G1, G2, frames_for, make_frames, shelf_layout  # noqa: E402
 
 
 def main():
@@ -47,6 +48,16 @@ def main():
     fr = synth.make_frame(9, small, H=576, W=832, inset=8, salt_p=0.02)
     insp.configure(Grid(boxes=[(b, i) for i, b in enumerate(small)]), is_reference=True)
     insp.inspect_batch(torch.from_numpy(fr[None]).cuda(), vi_b200.default_params(threshold=8, min_area=0, erode_px=1))
+    # ragged grids, many units of different sizes per CTA: the tensor-box gather (G1), the row-copy gather (G2), the
+    # general kernel (G1, blur 5 / morph 5) and the global arena (G1 plus a 640 x 480 unit)
+    for units, kws in ((G1, (dict(), dict(gaussian_blur=5, morph_kernel=5))), (G2, (dict(),)),
+                       (ARENA_UNITS, (dict(), dict(defect_method=1), dict(seg_method=1, adapt_block=11, adapt_C=5)))):
+        boxes, _, bottom = shelf_layout(units, 1008)
+        n = frames_for(len(units), torch.cuda.get_device_properties(0).multi_processor_count)
+        fr = make_frames(boxes, n, bottom + 8, 1024, 50)
+        insp.configure(Grid(boxes=boxes, exclusions=EXCL), is_reference=True)
+        for kw in kws:
+            insp.inspect_batch(torch.from_numpy(fr).cuda(), vi_b200.default_params(**kw))
     torch.cuda.synchronize()
     word = C.c_uint32(12345)
     _lib.check(insp._lib.vi_debug_check_word(insp._ctx, C.byref(word)))

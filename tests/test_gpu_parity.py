@@ -472,7 +472,7 @@ def test_calls_are_ordered_without_caller_synchronisation(insp, golden):
         assert torch.equal(seg, ref_seg) and torch.equal(dfm, ref_def) and torch.equal(rec, ref_rec)
 
 
-LARGE_UNITS = [(340, 340), (640, 480), (1000, 60), (2048, 1500)]
+LARGE_UNITS = [(360, 360), (640, 480), (1000, 60), (2048, 1500)]      # 360 x 360: a square just beyond one SM's shared memory
 
 
 @pytest.mark.parametrize("wh", LARGE_UNITS)
@@ -535,9 +535,10 @@ def test_unit_size_bound_is_documented_and_loud(insp):
     with pytest.raises(vi_b200.ViError) as e:
         insp.set_grid([(0, 0, 5000, 100)])
     assert e.value.code == -4
-    with pytest.raises(vi_b200.ViError) as e:
-        insp.set_grid([(0, 0, 4096, 4097)])
-    assert e.value.code == -4 and "bound" in str(e.value)
+    for rect in ((0, 0, 4096, 4097), (0, 0, 2049, 8192), (0, 0, 4097, 1), (0, 0, 1, 8193)):
+        with pytest.raises(vi_b200.ViError) as e:
+            insp.set_grid([(0, 0, 8, 8), rect])
+        assert e.value.code == -4 and "bound" in str(e.value), rect
 
 
 def test_config5_full_size_against_the_oracle(insp):

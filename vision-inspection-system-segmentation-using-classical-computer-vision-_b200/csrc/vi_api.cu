@@ -203,7 +203,9 @@ static int set_grid_state(vi_ctx* c, GridState& gs, const int32_t* r, int n, cud
     for (int i = 0; i < n; ++i) {
         int x = r[4 * i], y = r[4 * i + 1], w = r[4 * i + 2], h = r[4 * i + 3];
         if (w <= 0 || h <= 0 || x < 0 || y < 0) return fail(VI_ERR_ARG, "grid: rect %d = (%d,%d,%d,%d) is invalid", i, x, y, w, h);
-        if (w > kMaxUnitW || h > kMaxUnitH) return fail(VI_ERR_TOO_LARGE, "grid: rect %d is %dx%d: beyond the bound of a unit (%d wide, %d high)", i, w, h, kMaxUnitW, kMaxUnitH);
+        if (w > kMaxUnitW || h > kMaxUnitH || (long long)w * h > kMaxUnitPixels)
+            return fail(VI_ERR_TOO_LARGE, "grid: rect %d is %dx%d: beyond the bound of a unit (%d wide, %d high, %lld pixels)", i, w, h,
+                        kMaxUnitW, kMaxUnitH, kMaxUnitPixels);
         gs.rects[i] = make_int4(x, y, w, h);
         gs.off[i + 1] = gs.off[i] + (long long)w * h;
         gs.woff[i + 1] = gs.woff[i] + (long long)((w + 31) / 32) * h;
@@ -220,11 +222,13 @@ static int set_grid_state(vi_ctx* c, GridState& gs, const int32_t* r, int n, cud
     }
     gs.gmem = false;
     if (!make_plan(gs.wmax, gs.hmax, c->smem_optin, c->smem_static, &gs.plan, gray_need, words_need)) {
-        // larger than one SM's shared memory: same pipeline over a per-CTA arena in global memory
+        // larger than one SM's shared memory: same pipeline over a per-CTA arena in global memory.  The pixel bound
+        // holds per unit (checked above); a ragged grid's wmax x hmax may exceed it (a 4096 x 200 strip next to a
+        // 200 x 8000 column), and everything sized from wmax x hmax is 64-bit or within int range up to 4096 x 8192.
         gs.gmem = true;
         if (!make_plan_gmem(gs.wmax, gs.hmax, &gs.plan, gray_need, words_need))
-            return fail(VI_ERR_TOO_LARGE, "grid: units up to %d x %d exceed the bound of a unit (%d wide, %d high, %lld pixels)",
-                        gs.wmax, gs.hmax, kMaxUnitW, kMaxUnitH, kMaxUnitPixels);
+            return fail(VI_ERR_TOO_LARGE, "grid: units up to %d x %d exceed the bound of a unit (%d wide, %d high)",
+                        gs.wmax, gs.hmax, kMaxUnitW, kMaxUnitH);
     }
     int rc;
     if ((rc = gs.d_rects.ensure(sizeof(int4) * n))) return rc;

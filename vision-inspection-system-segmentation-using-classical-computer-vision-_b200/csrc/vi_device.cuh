@@ -167,12 +167,14 @@ __host__ inline bool make_plan(int wmax, int hmax, int smem_limit, int fixed, Sm
 // (L2-resident for mid-size units); only the lane-private histogram copies stay in shared memory.  `total` is the
 // dynamic shared memory (the histogram copies), the arena needs gray_bytes + kNumMasks * mask_bytes + ws_bytes.
 // Bounds of a unit: 255 * pixels must fit 32 bits (histogram moments), and the index arithmetic of the phases
-// (magic_div: n * d < 2^32) holds for w <= 4096, h <= 8192.  A whole 4096x3000 frame is a legal unit.
+// (magic_div: n * d < 2^32) holds for w <= 4096, h <= 8192.  A whole 4096x3000 frame is a legal unit.  The pixel bound
+// is a bound per unit (vi_api.cu: set_grid_state): a ragged grid's largest width and largest height, which size the
+// plan and the per-CTA scratch, may come from different units and multiply to more than 2^24.
 constexpr long long kMaxUnitPixels = 1ll << 24;
 constexpr int kMaxUnitW = 4096, kMaxUnitH = 8192;
 
 __host__ inline bool make_plan_gmem(int wmax, int hmax, SmemPlan* p, int gray_need, int mask_words_need) {
-    if ((long long)wmax * hmax > kMaxUnitPixels || wmax > kMaxUnitW || hmax > kMaxUnitH) return false;
+    if (wmax > kMaxUnitW || hmax > kMaxUnitH) return false;
     Geom g = make_geom(wmax, hmax);
     p->gray_bytes = align16(gray_need > 0 ? gray_need : g.gp * hmax);
     p->mask_bytes = align16((mask_words_need > 0 ? mask_words_need : g.nwords) * 4);
