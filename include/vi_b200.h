@@ -129,6 +129,24 @@ int vi_inspect_batch(vi_ctx* ctx, const uint8_t* d_frames, int n_images, int W, 
  * does).  d_stats: device, int64 [n_images*n_units][3]; NULL switches it off. */
 int vi_set_seg_stats_output(vi_ctx* ctx, int64_t* d_stats);
 
+/* One kept defect component: an external contour of the opened residual that passed the area filter
+ * (indexing_ui.py:1551-1558).  Unit-local coordinates, like the masks and vi_unit_record.cx / cy.  40 bytes. */
+typedef struct vi_defect_blob {
+    int32_t x, y, w, h;   /* bounding box = cv2.boundingRect(contour)                                        */
+    int32_t area;         /* pixels of the filled contour (drawContours FILLED): its share of defect_area     */
+    int32_t area2;        /* 2 * cv2.contourArea(contour), exact                                              */
+    double cx, cy;        /* mean x, mean y of those pixels (mask_stats of the filled contour)                */
+} vi_defect_blob;
+
+#define VI_MAX_BLOBS_PER_UNIT 1024
+
+/* Optional output of subsequent vi_inspect_batch calls, the table of kept defect components.  d_blobs: device,
+ * [n_images*n_units][max_per_unit].  Slot j of (image, unit) holds the j-th kept component in raster order of its
+ * first pixel, for j < min(n_kept, max_per_unit); later slots are not written.  vi_unit_record.n_kept stays the total.
+ * Units whose ROI is empty or whose residual does not survive the opening write none (n_kept is 0 there).
+ * max_per_unit outside 1..VI_MAX_BLOBS_PER_UNIT is VI_ERR_ARG; NULL switches the table off. */
+int vi_set_defect_blob_output(vi_ctx* ctx, vi_defect_blob* d_blobs, int max_per_unit);
+
 /* Same, from and to HOST buffers: works through the batch in chunks on internal
  * streams so that upload, compute and download overlap; blocks until done.  Pinned
  * and pageable frames take the same path: the frame rows that some unit covers are
@@ -150,6 +168,14 @@ int vi_inspect_batch_host_fmt(vi_ctx* ctx, const uint8_t* h_frames, int n_images
                               int64_t row_pitch, int64_t image_stride, const vi_params* params,
                               int mask_format, void* h_seg_masks, void* h_defect_masks,
                               vi_unit_record* h_records);
+
+/* vi_inspect_batch_host_fmt plus the kept-component table (vi_set_defect_blob_output) into a host buffer
+ * h_blobs [n_images*n_units][max_per_unit]; h_blobs NULL: none.  Here the slots past min(n_kept, max_per_unit)
+ * are unspecified (whole device tables are downloaded beside the records). */
+int vi_inspect_batch_host_blobs(vi_ctx* ctx, const uint8_t* h_frames, int n_images, int W, int H,
+                                int64_t row_pitch, int64_t image_stride, const vi_params* params,
+                                int mask_format, void* h_seg_masks, void* h_defect_masks,
+                                vi_unit_record* h_records, vi_defect_blob* h_blobs, int max_per_unit);
 
 /* Packed-bit masks (VI_MASKS_PACKED layout) as an optional extra output of subsequent vi_inspect_batch calls:
  * device pointers, vi_packed_mask_bytes per image; NULL switches one off. */

@@ -13,7 +13,7 @@ from typing import Optional, Sequence
 import numpy as np
 
 from . import _lib
-from ._lib import RECORD_DTYPE, ViExcl, check, default_params
+from ._lib import BLOB_DTYPE, RECORD_DTYPE, ViExcl, check, default_params
 from .grid import Grid, exclusions_to_table
 
 
@@ -100,10 +100,12 @@ class Inspector:
             raise ValueError(f"{name} holds {t.numel()} elements, the batch needs {numel}")
 
     def inspect_batch(self, frames, params=None, seg_masks=None, defect_masks=None, records=None, labels=None,
-                      stream=None, seg_stats=None, seg_bits=None, defect_bits=None):
+                      stream=None, seg_stats=None, seg_bits=None, defect_bits=None, defect_blobs=None):
         """frames: CUDA uint8 tensor [n, H, W] (row stride may exceed W).  Returns
         (records, seg_masks, defect_masks) as CUDA tensors (records: uint8 [n*units, 64]);
-        asynchronous on `stream` (default: torch's current stream)."""
+        asynchronous on `stream` (default: torch's current stream).
+        defect_blobs: optional CUDA uint8 [n*units, K, 40] (1 <= K <= 1024): row uid gets the first min(n_kept, K) kept
+        defect components of that unit (BLOB_DTYPE, raster order of their first pixel); later entries are not written."""
         import torch
         if not frames.is_cuda or frames.dtype != torch.uint8 or frames.dim() != 3:
             raise TypeError("frames must be a CUDA uint8 tensor [n, H, W]")
@@ -121,6 +123,12 @@ class Inspector:
         self._check_out(seg_stats, "seg_stats", dev, torch.int64, n * self.n_units * 3)
         self._check_out(seg_bits, "seg_bits", dev, torch.uint8, n * self.packed_bytes)
         self._check_out(defect_bits, "defect_bits", dev, torch.uint8, n * self.packed_bytes)
+        k_blobs = 0
+        if defect_blobs is not None:
+            if defect_blobs.dim() != 3 or defect_blobs.shape[2] != BLOB_DTYPE.itemsize:
+                raise ValueError(f"defect_blobs must be [n*units, K, {BLOB_DTYPE.itemsize}]")
+            k_blobs = int(defect_blobs.shape[1])
+            self._check_out(defect_blobs, "defect_blobs", dev, torch.uint8, n * self.n_units * k_blobs * BLOB_DTYPE.itemsize)
         if seg_masks is None:
             seg_masks = torch.empty(total, dtype=torch.uint8, device=dev)
         if defect_masks is None:
@@ -134,6 +142,8 @@ class Inspector:
         # seg_bits / defect_bits: optional CUDA uint8 [n * packed_bytes]: the masks as 1 bit per pixel (PNG scanline order)
         check(self._lib.vi_set_packed_mask_output(self._ctx, seg_bits.data_ptr() if seg_bits is not None else None,
                                                   defect_bits.data_ptr() if defect_bits is not None else None))
+        check(self._lib.vi_set_defect_blob_output(self._ctx, defect_blobs.data_ptr() if defect_blobs is not None else None,
+                                                  k_blobs))
         check(self._lib.vi_inspect_batch(
             self._ctx, frames.data_ptr(), int(n), int(W), int(H), int(frames.stride(1)),
             int(frames.stride(0)) if n > 1 else int(frames.stride(1)) * int(H),
@@ -176,11 +186,14 @@ class Inspector:
                                          C.c_void_p(st.cuda_stream)))
         return out
 
-    def inspect_batch_host(self, frames: np.ndarray, params=None, want_masks=True, out=None, mask_format="bytes"):
+    def inspect_batch_host(self, frames: np.ndarray, params=None, want_masks=True, out=None, mask_format="bytes",
+                           max_blobs=0):
         """frames: host uint8 [n, H, W] (numpy, pageable or pinned -- e.g. a torch pin_memory tensor's .numpy(); either
         way the rows the grid covers are copied to the device).  mask_format: "bytes" (0/255, the reference's masks), "packed"
         (1 bit per pixel, see `unpack_masks`) or "none" (records only).
-        Returns (records structured array, seg_masks u8 | None, defect_masks u8 | None)."""
+        Returns (records structured array, seg_masks u8 | None, defect_masks u8 | None).  With max_blobs = K > 0 a 4th
+        element follows: the kept defect components, BLOB_DTYPE [n, units, K], of which the first min(n_kept, K) of each
+        unit are valid (`kept_blobs`)."""
         frames = _u8c(frames, "frames")
         if frames.ndim != 3:
             raise ValueError("frames must be [n, H, W]")
@@ -204,11 +217,32 @@ class Inspector:
         if fmt == _lib.MASKS_NONE:
             seg = dfm = None
         p = params if params is not None else default_params()
+        if max_blobs:
+            if not 1 <= int(max_blobs) <= _lib.MAX_BLOBS_PER_UNIT:
+                raise ValueError(f"max_blobs must be in 1..{_lib.MAX_BLOBS_PER_UNIT}, got {max_blobs}")
+            blobs = np.empty((n, self.n_units, int(max_blobs)), BLOB_DTYPE)
+            check(self._lib.vi_inspect_batch_host_blobs(
+                self._ctx, frames.ctypes.data, int(n), int(W), int(H), int(W), int(H) * int(W), C.byref(p), fmt,
+                seg.ctypes.data if seg is not None else None, dfm.ctypes.data if dfm is not None else None,
+                rec.ctypes.data, blobs.ctypes.data, int(max_blobs)))
+            return rec, seg, dfm, blobs
         check(self._lib.vi_inspect_batch_host_fmt(
             self._ctx, frames.ctypes.data, int(n), int(W), int(H), int(W), int(H) * int(W), C.byref(p), fmt,
             seg.ctypes.data if seg is not None else None, dfm.ctypes.data if dfm is not None else None,
             rec.ctypes.data))
         return rec, seg, dfm
+
+    def kept_blobs(self, records, blobs, image, unit):
+        """The valid kept-component entries of one (image, unit): records (RECORD_DTYPE, [n*units] or [n, units]) and a
+        blob table from either batch call (BLOB_DTYPE [n, units, K], or the device table's uint8 [n*units, K, 40] copied
+        to the host).  Returns a BLOB_DTYPE array of min(n_kept, K) entries, unit-local coordinates."""
+        b = np.asarray(blobs)
+        if b.dtype != BLOB_DTYPE:
+            b = np.ascontiguousarray(b).view(BLOB_DTYPE)[..., 0]
+        uid = int(image) * self.n_units + int(unit)
+        b = b.reshape(-1, b.shape[-1])
+        n_kept = int(np.asarray(records).reshape(-1)[uid]['n_kept'])
+        return b[uid, :min(n_kept, b.shape[1])]
 
     def unpack_masks(self, packed, image=0):
         """One image's packed-bit mask block (mask_format="packed") as a list of (h, w) uint8 0/255 arrays."""

@@ -94,15 +94,18 @@ struct vi_ctx {
     long long scratch_stride = 0;
     long long scratch_f32_off = 0;
     long long scratch_rank_off = 0;
+    long long scratch_blob_off = 0;
     // compat / host-batch staging
     DevBuf st_in, st_aux, st_out, st_out2, st_rec, st_stats, st_lab;
-    DevBuf hb_frames[kHostSlots], hb_seg[kHostSlots], hb_def[kHostSlots], hb_rec[kHostSlots];
+    DevBuf hb_frames[kHostSlots], hb_seg[kHostSlots], hb_def[kHostSlots], hb_rec[kHostSlots], hb_blob[kHostSlots];
     cudaStream_t streams[kHostSlots] = {};
     int smem_set = 0;
     long long* prof = nullptr;
     long long* seg_stats = nullptr;
     uint32_t* seg_bits = nullptr;   // optional packed-bit outputs of vi_inspect_batch (vi_set_packed_mask_output)
     uint32_t* def_bits = nullptr;
+    vi_defect_blob* blobs = nullptr;   // optional kept-component table of vi_inspect_batch (vi_set_defect_blob_output)
+    int blob_k = 0;
     // Ordering: the context's tables and per-CTA scratch are shared by every call.  `busy` is recorded after each
     // asynchronous launch on a caller's stream; every later entry point waits on it (streams: cudaStreamWaitEvent,
     // host-side table updates: cudaEventSynchronize) before it touches them.
@@ -185,7 +188,7 @@ extern "C" void vi_ctx_destroy(vi_ctx* c) {
                       &c->st_stats, &c->st_lab})
         b->release();
     for (int i = 0; i < kHostSlots; ++i) {
-        c->hb_frames[i].release(); c->hb_seg[i].release(); c->hb_def[i].release(); c->hb_rec[i].release();
+        c->hb_frames[i].release(); c->hb_seg[i].release(); c->hb_def[i].release(); c->hb_rec[i].release(); c->hb_blob[i].release();
         if (c->streams[i]) cudaStreamDestroy(c->streams[i]);
     }
     delete c;
@@ -355,6 +358,15 @@ extern "C" int vi_debug_set_profile(vi_ctx* c, long long* d_cycles) {
 extern "C" int vi_set_seg_stats_output(vi_ctx* c, int64_t* d_stats) {
     if (!c) return fail(VI_ERR_ARG, "ctx is null");
     c->seg_stats = (long long*)d_stats;
+    return VI_OK;
+}
+
+extern "C" int vi_set_defect_blob_output(vi_ctx* c, vi_defect_blob* d_blobs, int max_per_unit) {
+    if (!c) return fail(VI_ERR_ARG, "ctx is null");
+    if (d_blobs && (max_per_unit < 1 || max_per_unit > VI_MAX_BLOBS_PER_UNIT))
+        return fail(VI_ERR_ARG, "vi_set_defect_blob_output: %d blobs per unit (1..%d)", max_per_unit, VI_MAX_BLOBS_PER_UNIT);
+    c->blobs = d_blobs;
+    c->blob_k = d_blobs ? max_per_unit : 0;
     return VI_OK;
 }
 
@@ -570,7 +582,7 @@ static int fill_params(KArgs& a, const vi_params* p) {
     return VI_OK;
 }
 
-static long long scratch_layout(vi_ctx* c, int wmax, int hmax, bool f32_plane) {
+static long long scratch_layout(vi_ctx* c, int wmax, int hmax, bool f32_plane, int blob_k) {
     long long px = (long long)wmax * hmax;
     long long capg = (long long)hmax * (wmax / 2 + 1);
     long long px4 = (long long)((wmax + 3) & ~3) * hmax;
@@ -580,6 +592,8 @@ static long long scratch_layout(vi_ctx* c, int wmax, int hmax, bool f32_plane) {
     stride += (rank_scratch_bytes(wmax, hmax) + 255) & ~255ll;
     c->scratch_f32_off = stride;
     if (f32_plane) stride += (px * 4 + 255) & ~255ll;       // float plane of the adaptive mean, only when asked for
+    c->scratch_blob_off = stride;
+    stride += ((long long)blob_k * sizeof(BlobAcc) + 255) & ~255ll;   // blob accumulators that do not fit two masks
     c->scratch_stride = stride;
     return stride;
 }
@@ -645,7 +659,7 @@ static int launch_units(vi_ctx* c, KArgs& a, const GridState& gs, cudaStream_t s
     if (n_total <= 0) return VI_OK;
     if (n_total > 0x7fffffffll) return fail(VI_ERR_ARG, "too many units in one call");
     int rc;
-    const long long stride = scratch_layout(c, gs.wmax, gs.hmax, a.p.seg_method == 1);
+    const long long stride = scratch_layout(c, gs.wmax, gs.hmax, a.p.seg_method == 1, a.blobs ? a.blob_k : 0);
     const long long astride = gs.gmem ? plan_arena_bytes(gs.plan) : 0;
     // CTAs per slot: one per SM; fewer when the units are so large that their scratch would not fit the budget
     int bps = c->sm_count;
@@ -658,6 +672,7 @@ static int launch_units(vi_ctx* c, KArgs& a, const GridState& gs, cudaStream_t s
     a.scratch_stride = stride;
     a.scratch_f32_off = c->scratch_f32_off;
     a.scratch_rank_off = c->scratch_rank_off;
+    a.scratch_blob_off = c->scratch_blob_off;
     a.arena = gs.gmem ? (uint8_t*)c->arena.p + (size_t)slot * bps * astride : nullptr;
     a.arena_stride = astride;
     a.wmax = gs.wmax; a.hmax = gs.hmax;
@@ -748,6 +763,7 @@ extern "C" int vi_inspect_batch(vi_ctx* c, const uint8_t* d_frames, int n_images
     a.seg_out = d_seg; a.def_out = d_def; a.labels_out = d_labels; a.rec = d_rec;
     a.seg_stats = c->seg_stats;
     a.seg_bits = c->seg_bits; a.def_bits = c->def_bits;
+    a.blobs = c->blobs; a.blob_k = c->blob_k;
     a.n_peers = c->n_peers; a.image_mul = c->image_mul; a.image_base = c->image_add;
     for (int i = 0; i < c->n_peers; ++i) a.peer_rec[i] = c->peer_rec[i];
     if ((rc = wait_busy_stream(c, (cudaStream_t)stream))) return rc;     // an earlier batch on another stream shares the scratch
@@ -759,11 +775,14 @@ extern "C" int vi_inspect_batch(vi_ctx* c, const uint8_t* d_frames, int n_images
 // VI_MASKS_PACKED (1 bit per pixel, rows of 32-bit words, PNG bit order) or VI_MASKS_NONE (records only: all that
 // run_inspection needs, indexing_ui.py:1686-1706).
 static int host_batch(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, int H, int64_t row_pitch, int64_t image_stride,
-                      const vi_params* params, int mask_format, void* h_seg, void* h_def, vi_unit_record* h_rec) {
+                      const vi_params* params, int mask_format, void* h_seg, void* h_def, vi_unit_record* h_rec,
+                      vi_defect_blob* h_blobs = nullptr, int blob_k = 0) {
     if (!c) return fail(VI_ERR_ARG, "ctx is null");
     if (c->grid.rects.empty()) return fail(VI_ERR_ARG, "vi_inspect_batch_host: no grid set");
     if (!h_frames || !h_rec) return fail(VI_ERR_ARG, "vi_inspect_batch_host: frames / records pointer is null");
     if (mask_format < VI_MASKS_BYTES || mask_format > VI_MASKS_NONE) return fail(VI_ERR_ARG, "mask_format %d", mask_format);
+    if (h_blobs && (blob_k < 1 || blob_k > VI_MAX_BLOBS_PER_UNIT))
+        return fail(VI_ERR_ARG, "vi_inspect_batch_host_blobs: %d blobs per unit (1..%d)", blob_k, VI_MAX_BLOBS_PER_UNIT);
     VI_DEVICE(c);
     int rc;
     if (n_images == 1 && image_stride < row_pitch * (int64_t)H) image_stride = row_pitch * (int64_t)H;   // one frame: the stride is moot
@@ -787,6 +806,7 @@ static int host_batch(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, i
         if (h_seg && (rc = c->hb_seg[b].ensure((size_t)ubytes * chunk))) return rc;
         if (h_def && (rc = c->hb_def[b].ensure((size_t)ubytes * chunk))) return rc;
         if ((rc = c->hb_rec[b].ensure(sizeof(vi_unit_record) * (size_t)n_units * chunk))) return rc;
+        if (h_blobs && (rc = c->hb_blob[b].ensure(sizeof(vi_defect_blob) * (size_t)n_units * chunk * blob_k))) return rc;
     }
     // Upload: one strided copy per covered row interval into the slot's staging buffer (the copy engine moves whole
     // frame rows at the link rate).
@@ -811,12 +831,17 @@ static int host_batch(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, i
                 a.seg_bits = h_seg ? (uint32_t*)c->hb_seg[slot].p : nullptr; a.def_bits = h_def ? (uint32_t*)c->hb_def[slot].p : nullptr;
             }
             a.rec = (vi_unit_record*)c->hb_rec[slot].p;
+            if (h_blobs) { a.blobs = (vi_defect_blob*)c->hb_blob[slot].p; a.blob_k = blob_k; }
             int r2;
             if ((r2 = launch_units(c, a, c->grid, st, slot))) return r2;
             if (h_seg) CU(cudaMemcpyAsync((uint8_t*)h_seg + (size_t)i0 * ubytes, c->hb_seg[slot].p, (size_t)ubytes * n, cudaMemcpyDeviceToHost, st));
             if (h_def) CU(cudaMemcpyAsync((uint8_t*)h_def + (size_t)i0 * ubytes, c->hb_def[slot].p, (size_t)ubytes * n, cudaMemcpyDeviceToHost, st));
             CU(cudaMemcpyAsync(h_rec + (size_t)i0 * n_units, c->hb_rec[slot].p, sizeof(vi_unit_record) * (size_t)n_units * n,
                                cudaMemcpyDeviceToHost, st));
+            // the whole slot table: entries past min(n_kept, blob_k) are unspecified
+            if (h_blobs)
+                CU(cudaMemcpyAsync(h_blobs + (size_t)i0 * n_units * blob_k, c->hb_blob[slot].p,
+                                   sizeof(vi_defect_blob) * (size_t)n_units * n * blob_k, cudaMemcpyDeviceToHost, st));
         }
         return VI_OK;
     };
@@ -839,6 +864,13 @@ extern "C" int vi_inspect_batch_host_fmt(vi_ctx* c, const uint8_t* h_frames, int
                                          int64_t image_stride, const vi_params* params, int mask_format, void* h_seg,
                                          void* h_def, vi_unit_record* h_rec) {
     return host_batch(c, h_frames, n_images, W, H, row_pitch, image_stride, params, mask_format, h_seg, h_def, h_rec);
+}
+
+extern "C" int vi_inspect_batch_host_blobs(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, int H, int64_t row_pitch,
+                                           int64_t image_stride, const vi_params* params, int mask_format, void* h_seg,
+                                           void* h_def, vi_unit_record* h_rec, vi_defect_blob* h_blobs, int max_per_unit) {
+    return host_batch(c, h_frames, n_images, W, H, row_pitch, image_stride, params, mask_format, h_seg, h_def, h_rec,
+                      h_blobs, max_per_unit);
 }
 
 // ---------------------------------------------------------------------------

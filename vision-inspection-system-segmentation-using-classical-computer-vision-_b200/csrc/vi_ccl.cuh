@@ -457,6 +457,64 @@ VI_PHASE void ccl_paint(unsigned* dst, const unsigned* base, const Geom& g, cons
     }
 }
 
+// Accumulator of one kept component of the defect-blob table (vi_set_defect_blob_output): pixel area, bounding box
+// and coordinate sums over its runs; ymin is the root run's row, area2 the area filter's acc0.
+struct BlobAcc {
+    unsigned long long sx, sy;
+    unsigned area, xmin, xmax, ymin, ymax, area2;
+};
+static_assert(sizeof(BlobAcc) == 40, "BlobAcc layout");
+
+// The first kc kept components of a labelling (after ccl_build and the per-root acc0 of the area filter), in raster
+// order of their first pixel, into out[0..kc).  acc1[root] = 1 + slot (an exclusive count of kept roots in increasing
+// run id, which is raster order); ccl_build left acc1 zero on every run, and 0 marks a root without a slot, so the
+// count stops at the kc-th kept root.  tab: kc accumulators (tab_cap of them fit).  Every thread reaches every barrier.
+template <class Keep>
+VI_PHASE void ccl_blob_table(Cta& cs, const CclWs& ws, int R, Keep keep, int kc, int tab_cap, BlobAcc* tab,
+                             vi_defect_blob* __restrict__ out) {
+    unsigned carry = 0;
+    for (int base = 0; base < R && (int)carry < kc; base += kThreads) {
+        const int i = base + threadIdx.x + 1;
+        const bool kept = i <= R && ws.parent()[i] == i && keep(i);
+        unsigned a = kept ? 1u : 0u, b = 0, ta, tb;
+        cta_excl_scan2(cs, a, b, ta, tb);
+        const unsigned s = carry + a;
+        if (kept && (int)s < kc) {
+            VI_CHECK((int)s < tab_cap, CHK_BLOB_SLOT);
+            ws.acc1()[i] = s + 1;
+            BlobAcc e;
+            e.sx = 0; e.sy = 0; e.area = 0; e.xmin = 0xffffffffu; e.xmax = 0; e.ymin = ws.yy()[i]; e.ymax = 0; e.area2 = ws.acc0()[i];
+            tab[s] = e;
+        }
+        carry += ta;
+    }
+    cta_sync();
+    for (int i = 1 + threadIdx.x; i <= R; i += kThreads) {
+        const unsigned s = ws.acc1()[ws.parent()[i]] - 1u;        // (no slot: 0xffffffff)
+        if (s < (unsigned)kc) {
+            VI_CHECK((int)s < tab_cap, CHK_BLOB_SLOT);
+            const unsigned xs = ws.xs()[i], xe = ws.xe()[i], y = ws.yy()[i], len = xe - xs + 1;
+            BlobAcc& e = tab[s];
+            atomicAdd(&e.area, len);
+            atomicMin(&e.xmin, xs);
+            atomicMax(&e.xmax, xe);
+            atomicMax(&e.ymax, y);
+            atomicAdd(&e.sx, (unsigned long long)(xs + xe) * len / 2);
+            atomicAdd(&e.sy, (unsigned long long)y * len);
+        }
+    }
+    cta_sync();
+    for (int j = threadIdx.x; j < kc; j += kThreads) {
+        const BlobAcc e = tab[j];
+        vi_defect_blob o;
+        o.x = (int)e.xmin; o.y = (int)e.ymin; o.w = (int)(e.xmax - e.xmin + 1); o.h = (int)(e.ymax - e.ymin + 1);
+        o.area = (int)e.area; o.area2 = (int)e.area2;
+        o.cx = __ddiv_rn((double)e.sx, (double)e.area);              // the record's centroid convention
+        o.cy = __ddiv_rn((double)e.sy, (double)e.area);
+        out[j] = o;
+    }
+}
+
 // rows 0..h-1 need row_first for every row, including rows without runs.
 // ccl_build writes row_first[y] only from the thread that owns word (y,0), which
 // exists for every row, so the table is always complete.

@@ -32,6 +32,7 @@ __device__ unsigned g_vi_check_word = 0;
 enum CheckCode : unsigned {
     CHK_BAND_LIST = 1, CHK_RUN_INDEX = 2, CHK_RUN_CAP = 3, CHK_UF_PARENT = 4, CHK_DIRTY_LIST = 5, CHK_EXACT_LIST = 6,
     CHK_LATTICE_SLOT = 7, CHK_HIST_COUNTER = 8, CHK_ROW_TABLE = 9, CHK_PAINT_RUN = 10, CHK_GATHER_STAGE = 11,
+    CHK_BLOB_SLOT = 12,
 };
 
 // Pipeline phases.  (Compiling them as __noinline__ functions of their own was measured: reference
@@ -244,6 +245,9 @@ struct KArgs {
     uint8_t* arena;                 // GMEM kernel: per-CTA global arena holding what the shared-memory plan holds
     long long arena_stride;         //  (gray crop, masks, workspace) for units larger than one SM's shared memory
     long long* prof;                // diagnostics: [n_total][kProfSlots] per-phase cycle counts, or null
+    vi_defect_blob* blobs;          // optional: [n_total][blob_k] kept defect components (vi_set_defect_blob_output), or null
+    int blob_k;
+    long long scratch_blob_off;     // offset of the blob accumulators inside a CTA's scratch (tables beyond two masks)
     SmemPlan plan;
     // Asynchronous crop gather through the tensor-memory accelerator (vi_pipeline.cuh: gather_issue_tma): the frames as
     // a 3-D uint8 tensor (x, y, image); one box = tma_bw x tma_bh pixels, a crop = tma_ncb x tma_nrb boxes that land as

@@ -628,7 +628,16 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
     const int n_kept = (int)cta_sum_u64(cta, kept);
     ccl_paint(ME, nullptr, g, ws, keep);
     cta_sync();
-    pt.tick();   // 14 component area filter
+    if (a.blobs && n_kept > 0) {
+        // the kept components as a table (vi_set_defect_blob_output): a run-time pointer, in every instantiation.  Its
+        // accumulators take MC and MD, dead from here on (MB was read by the area pass above, MA may be receiving the
+        // next unit's crop; in GMEM they are the arena's), or the CTA's global scratch when they do not fit there.
+        const int kc = min(n_kept, a.blob_k);
+        const int cap_m = 2 * plan.mask_bytes / (int)sizeof(BlobAcc);
+        BlobAcc* tab = kc <= cap_m ? reinterpret_cast<BlobAcc*>(MC) : reinterpret_cast<BlobAcc*>(gs + a.scratch_blob_off);
+        ccl_blob_table(cta, ws, R, keep, kc, kc <= cap_m ? cap_m : a.blob_k, tab, a.blobs + (long long)uid * a.blob_k);
+    }
+    pt.tick();   // 14 component area filter (+ blob table)
     // ---- P14: verdict ---------------------------------------------------------
     const unsigned defect_area = cta_popcount(cta, ME, g);
     if (def_out) store_mask_bytes_sparse(ME, g, def_out);
