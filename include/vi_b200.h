@@ -251,6 +251,10 @@ int vi_debug_check_word(vi_ctx* ctx, uint32_t* out_code);
 /* Compares the reciprocal-based division of the Otsu recurrence with the IEEE divide on
  * n_samples pseudo-random operand pairs; *mismatches must come back 0. */
 int vi_debug_fastdiv_check(vi_ctx* ctx, long long n_samples, unsigned long long seed, long long* mismatches);
+/* The device Otsu threshold of n histograms (device memory: d_hists [n][256], d_npix [n] = each one's pixel count,
+ * 1..2^24): d_out [n][3] = t (the exact scan, cv2.threshold's OTSU value), t_apx (the float32 arg max) and last (the
+ * bound the scan stops at).  VI_ERR_ARG (and -1 in that row) when an npix is out of range or not its histogram's sum. */
+int vi_debug_otsu(vi_ctx* ctx, const uint32_t* d_hists, const int* d_npix, int n, int* d_out);
 
 /* Host only: the float32 taps of the adaptive threshold's Gaussian mean for an odd block size
  * (cv2.getGaussianKernel(bs, 0, CV_32F) as cv2.adaptiveThreshold uses it, segmentation.py:85). */

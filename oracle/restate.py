@@ -117,6 +117,80 @@ def otsu_from_hist(hist) -> int:
     return max_val
 
 
+def _otsu_scan_rows(H, last=None):
+    """otsu_from_hist on every row of H, scoring only bins <= last (per row) when given."""
+    H = np.asarray(H, dtype=np.int64)
+    Hf = np.ascontiguousarray(H.T).astype(np.float64)          # [256, n]: exact (counts < 2^53)
+    n = H.shape[0]
+    scale = 1.0 / Hf.sum(0)
+    mu = np.zeros(n)
+    for i in range(256):
+        mu += i * Hf[i]
+    mu *= scale
+    mu1 = np.zeros(n)
+    q1 = np.zeros(n)
+    max_sigma = np.zeros(n)
+    max_val = np.zeros(n, np.int64)
+    with np.errstate(divide='ignore', invalid='ignore'):
+        for i in range(256):
+            p_i = Hf[i] * scale
+            mu1 *= q1
+            q1 = q1 + p_i
+            q2 = 1.0 - q1
+            ok = ~((np.minimum(q1, q2) < FLT_EPSILON) | (np.maximum(q1, q2) > 1.0 - FLT_EPSILON))
+            if last is not None:
+                ok &= i <= last
+            m1 = (mu1 + i * p_i) / q1
+            mu2 = (mu - q1 * m1) / q2
+            sigma = q1 * q2 * (m1 - mu2) * (m1 - mu2)
+            mu1 = np.where(ok, m1, mu1)
+            better = ok & (sigma > max_sigma)
+            max_sigma = np.where(better, sigma, max_sigma)
+            max_val = np.where(better, i, max_val)
+    return max_val
+
+
+def otsu_from_hists(H) -> np.ndarray:
+    """otsu_from_hist over the rows of H ([n, 256] counts, each row's sum >= 1), vectorised: the same float64
+    operations in the same order on every row, so the same thresholds bit for bit."""
+    return _otsu_scan_rows(H)
+
+
+def otsu_kernel_model(H, slack: float = 0.0):
+    """The two steps of the device Otsu (vi_pipeline.cuh) on the rows of H ([n, 256] counts, sums 1..2^24):
+    otsu_approx_warp's float32 between-class variances from exact integer moments (IEEE division where the kernel
+    uses __fdividef) give `last`, the last bin within 2e-5 of their maximum; otsu_scan is the reference scan scoring
+    bins <= last only.  Bins whose lower class is below FLT_EPSILON of the pixels (n1 * 2^23 < N), which the
+    reference skips, score 0, as do bins with an empty upper class.  Once the reference skips a lone darkest pixel
+    at x0, its mu1 lacks that pixel's x0 / N for good, so every later variance is the one of lower-class moment
+    m1 - x0.  slack > 0 lowers every variance by that fraction and raises the maximum by as much, so `last` is what a
+    division off by that much could give at worst.
+    Returns (t, last), int64 arrays."""
+    H = np.asarray(H, dtype=np.int64)
+    N = H.sum(1)[:, None]
+    n1 = np.cumsum(H, 1)
+    m1 = np.cumsum(H * np.arange(256), 1)
+    n2 = N - n1
+    # above 2^23 pixels a lone darkest pixel's split is skipped, and with it the step that adds its value to mu1
+    x0 = np.argmax(H > 0, 1)[:, None]
+    drop = np.where((np.take_along_axis(H, x0, 1) == 1) & (N > (1 << 23)), x0, 0)
+    dd = m1[:, -1:] * n1 - N * (m1 - drop)                      # exact: |dd| < 2^56
+    f = dd.astype(np.float32)
+    den = n1.astype(np.float32) * n2.astype(np.float32)
+    scored = ((n1 << 23) >= N) & (n2 > 0)
+    with np.errstate(divide='ignore', invalid='ignore'):
+        v = np.where(scored, (f * f) / den, np.float32(0))
+    mx = v.max(1, keepdims=True)
+    keep = np.float32(1) - np.float32(2e-5)
+    if slack:
+        ge = v.astype(np.float64) * (1.0 - slack) >= mx.astype(np.float64) * (1.0 + slack) * np.float64(keep)
+    else:
+        ge = v >= mx * keep
+    lc = 255 - np.argmax(ge[:, ::-1], 1)
+    last = np.where(mx[:, 0] > 0, lc, 255)
+    return _otsu_scan_rows(H, last), last
+
+
 def otsu_inv_mask(img) -> Tuple[int, np.ndarray]:
     t = otsu_from_hist(np.bincount(img.ravel(), minlength=256))
     return t, np.where(img > t, 0, 255).astype(np.uint8)

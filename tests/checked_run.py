@@ -58,6 +58,15 @@ def main():
         insp.configure(Grid(boxes=boxes, exclusions=EXCL), is_reference=True)
         for kw in kws:
             insp.inspect_batch(torch.from_numpy(fr).cuda(), vi_b200.default_params(**kw))
+    # the device Otsu on its own: adversarial histograms, two with a bad pixel count (VI_ERR_ARG, rows of -1)
+    import otsu_families as F
+    H, _ = F.mixed(rng, 500)
+    npix = H.sum(1)
+    npix[:2] = (0, (1 << 24) + 1)
+    out = torch.empty((len(H), 3), dtype=torch.int32, device="cuda")
+    dh = torch.from_numpy(H.astype(np.uint32).view(np.int32)).cuda()
+    dn = torch.from_numpy(npix.astype(np.int32)).cuda()
+    assert insp._lib.vi_debug_otsu(insp._ctx, dh.data_ptr(), dn.data_ptr(), len(H), out.data_ptr()) == _lib.VI_ERR_ARG
     torch.cuda.synchronize()
     word = C.c_uint32(12345)
     _lib.check(insp._lib.vi_debug_check_word(insp._ctx, C.byref(word)))

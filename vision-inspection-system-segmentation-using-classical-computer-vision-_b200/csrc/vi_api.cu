@@ -334,6 +334,59 @@ extern "C" int vi_debug_fastdiv_check(vi_ctx* c, long long n_samples, unsigned l
     return VI_OK;
 }
 
+// Diagnostics: the device Otsu of arbitrary histograms, one 2-warp CTA each.  Warp 0 runs otsu_approx_warp and
+// publishes the bound before the barrier, so otsu_scan on warp 1 always finds it (the inspection kernel runs the two
+// concurrently).  out[3b .. 3b+2] = t, t_apx, last; -1 for a histogram whose npix is outside 1..2^24 or not its sum.
+__global__ void otsu_debug_kernel(const uint32_t* hists, const int* npix, int* out, unsigned* bad) {
+    __shared__ unsigned hist[256];
+    __shared__ __align__(16) double ws[vi::kOtsuWsBytes / 8];
+    __shared__ int last_s, tapx_s, ok_s;
+    const long long b = blockIdx.x;
+    for (int i = threadIdx.x; i < 256; i += blockDim.x) hist[i] = hists[b * 256 + i];
+    __syncthreads();
+    const int N = npix[b];
+    if (threadIdx.x < 32) {
+        unsigned long long s = 0;
+        for (int i = threadIdx.x; i < 256; i += 32) s += hist[i];
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) s += __shfl_xor_sync(vi::kFull, s, o);
+        if (threadIdx.x == 0) { ok_s = N >= 1 && N <= (1 << 24) && s == (unsigned long long)N; last_s = -1; }
+    }
+    __syncthreads();
+    if (!ok_s) {
+        if (threadIdx.x == 0) { out[3 * b] = out[3 * b + 1] = out[3 * b + 2] = -1; atomicAdd(bad, 1u); }
+        return;
+    }
+    vi::PhaseTimerT<false> pt;
+    if (threadIdx.x < 32) {
+        int last;
+        const int ta = vi::otsu_approx_warp(hist, N, last);
+        if (threadIdx.x == 0) { tapx_s = ta; last_s = last; }
+    }
+    __syncthreads();
+    if (threadIdx.x >= 32) {
+        const int t = vi::otsu_scan(hist, N, ws, &last_s, pt);
+        if (threadIdx.x == 32) { out[3 * b] = t; out[3 * b + 1] = tapx_s; out[3 * b + 2] = last_s; }
+    }
+}
+
+extern "C" int vi_debug_otsu(vi_ctx* c, const uint32_t* d_hists, const int* d_npix, int n, int* d_out) {
+    if (!c || n < 0 || (n > 0 && (!d_hists || !d_npix || !d_out))) return fail(VI_ERR_ARG, "vi_debug_otsu: null or n < 0");
+    if (n == 0) return VI_OK;
+    VI_DEVICE(c);
+    unsigned* d_bad = nullptr;
+    CU(cudaMalloc(&d_bad, 4));
+    CU(cudaMemset(d_bad, 0, 4));
+    otsu_debug_kernel<<<n, 64>>>(d_hists, d_npix, d_out, d_bad);
+    unsigned h = 0;
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpy(&h, d_bad, 4, cudaMemcpyDeviceToHost);
+    cudaFree(d_bad);
+    if (e != cudaSuccess) return fail(VI_ERR_CUDA, "vi_debug_otsu: %s", cudaGetErrorString(e));
+    if (h) return fail(VI_ERR_ARG, "vi_debug_otsu: %u histograms whose npix is outside 1..2^24 or differs from their sum", h);
+    return VI_OK;
+}
+
 extern "C" int vi_debug_check_word(vi_ctx* c, uint32_t* out) {
     if (!c || !out) return fail(VI_ERR_ARG, "vi_debug_check_word: null");
 #ifdef VI_CHECKED
