@@ -255,6 +255,15 @@ int vi_debug_fastdiv_check(vi_ctx* ctx, long long n_samples, unsigned long long 
  * 1..2^24): d_out [n][3] = t (the exact scan, cv2.threshold's OTSU value), t_apx (the float32 arg max) and last (the
  * bound the scan stops at).  VI_ERR_ARG (and -1 in that row) when an npix is out of range or not its histogram's sum. */
 int vi_debug_otsu(vi_ctx* ctx, const uint32_t* d_hists, const int* d_npix, int n, int* d_out);
+/* The median residual stage alone (|gray - medianBlur(gray, 21)| > thr inside the ROI), one CTA running the inspection
+ * kernel's device functions on caller-chosen levels (host int[3], sorted, 0..255) instead of its own.  Device memory:
+ * d_gray [h][w] and d_roi [h][w] (non-zero = inside), w x h inside the unit bound; d_cand receives the raw candidate
+ * mask, h rows of (w + 31) / 32 words, bit x & 31 of word x >> 5 (padding bits 0).  thr and pad (the byte written past w
+ * in each row of the kernel's crop copy) in 0..255; ccap in 0..4096 and ecap in 0..16384 cap the dirty-cell and the
+ * ambiguous-pixel lists (the rest take the inline overflow paths).  Host counts[3] = ambiguous-pixel list entries (one
+ * per open test), dirty cells that touch the ROI, the exact Otsu threshold of the crop's histogram. */
+int vi_debug_rank_residual(vi_ctx* ctx, const uint8_t* d_gray, const uint8_t* d_roi, int w, int h, const int* levels, int thr,
+                           int ccap, int ecap, int pad, uint32_t* d_cand, int* counts);
 
 /* Host only: the float32 taps of the adaptive threshold's Gaussian mean for an odd block size
  * (cv2.getGaussianKernel(bs, 0, CV_32F) as cv2.adaptiveThreshold uses it, segmentation.py:85). */

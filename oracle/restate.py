@@ -407,35 +407,79 @@ def residual_mask_rank(gray, thr: int, levels, stats: Optional[dict] = None):
     return out
 
 
-def residual_mask_lattice(gray, thr: int, levels, roi=None, stats: Optional[dict] = None):
+def _lattice_brackets(gray, thr: int, levels):
+    """C_k at the cell centres ([K][ny][nx]) and each cell's bracket LO < med <= HI ([ny][nx])."""
+    K = len(levels)
+    h, w = gray.shape
+    ny, nx = (h + 2) // 3, (w + 2) // 3
+    # exact counts at virtual centres (3j+1, 3i+1): replicate padding also beyond the crop
+    pad = np.pad(gray, ((10, 10 + 3), (10, 10 + 3)), mode='edge')
+    cy = 3 * np.arange(ny) + 1
+    cx = 3 * np.arange(nx) + 1
+    centre = []
+    for v in levels:
+        ind = (pad <= v).astype(np.int32)
+        s = np.pad(np.cumsum(np.cumsum(ind, axis=0), axis=1), ((1, 0), (1, 0)))
+        centre.append(s[cy[:, None] + 21, cx[None, :] + 21] - s[cy[:, None], cx[None, :] + 21]
+                      - s[cy[:, None] + 21, cx[None, :]] + s[cy[:, None], cx[None, :]])
+    C = np.stack(centre)
+    lo_idx = (C <= 178).sum(0)
+    hi_idx = K - (C >= 263).sum(0)
+    LO = np.array([-1] + levels, np.int32)[lo_idx]
+    HI = np.array(levels + [255], np.int32)[hi_idx]
+    return C, LO, HI
+
+
+def lattice_stats(gray, thr: int, levels, roi=None, cell_gray=None) -> dict:
+    """What the kernel's stage counts (vi_rank.cuh: rank_dirty_cell, rank_finish), from the twin's brackets:
+      ambiguous        ambiguous pixels (of the ROI when one is given): neither defect nor clean for sure
+      entries          list entries, one per open test of an ambiguous pixel:
+                       [g < HI - thr] + [g > LO + thr + 1]
+      centre_counts    [K][ny][nx] C_k at the cell centres
+      dirty_roi_cells  cells whose gray min or max leaves the clean range [HI - thr, LO + thr + 1]
+                       and that hold a ROI pixel (every such cell without a ROI)
+      codes            [16] bracket codes n179 * 4 + n263 of those cells (n263 <= n179: ten occur)
+    The cell min / max are taken over `cell_gray` ([3 ny][3 nx], the bytes the kernel's min / max pass reads)
+    when given, else over the crop with replicated rows and columns."""
+    levels = sorted(int(v) for v in levels)
+    h, w = gray.shape
+    ny, nx = (h + 2) // 3, (w + 2) // 3
+    C, LO, HI = _lattice_brackets(gray, thr, levels)
+    g = gray.astype(np.int32)
+    LOp = np.repeat(np.repeat(LO, 3, axis=0), 3, axis=1)[:h, :w]
+    HIp = np.repeat(np.repeat(HI, 3, axis=0), 3, axis=1)[:h, :w]
+    sure = (g <= LOp - thr) | (g >= HIp + thr + 1)
+    ta, tb = g < HIp - thr, g > LOp + thr + 1
+    amb = ~sure & (ta | tb)
+    if roi is not None:
+        amb &= roi
+    if cell_gray is None:
+        cell_gray = np.pad(gray, ((0, 3 * ny - h), (0, 3 * nx - w)), mode='edge')
+    cg = cell_gray[:3 * ny, :3 * nx].astype(np.int32).reshape(ny, 3, nx, 3)
+    dirty = (cg.min(axis=(1, 3)) < HI - thr) | (cg.max(axis=(1, 3)) > LO + thr + 1)
+    if roi is not None:
+        rp = np.pad(np.asarray(roi, bool), ((0, 3 * ny - h), (0, 3 * nx - w)))
+        dirty &= rp.reshape(ny, 3, nx, 3).any(axis=(1, 3))
+    code = (C >= 179).sum(0) * 4 + (C >= 263).sum(0)
+    return dict(ambiguous=int(amb.sum()), entries=int((amb & ta).sum() + (amb & tb).sum()), centre_counts=C,
+                dirty_roi_cells=int(dirty.sum()), codes=np.bincount(code[dirty], minlength=16),
+                amb=amb, ta=ta, tb=tb)
+
+
+def residual_mask_lattice(gray, thr: int, levels, roi=None, stats: Optional[dict] = None, cell_gray=None):
     """numpy twin of the CUDA rank-count stage (csrc/vi_rank.cuh): exact window
     counts only at the centre of every 3x3 cell; |C(p) - C(q)| <= 21 * L1(p, q)
     <= 42 inside a cell, so C(centre) >= 263 proves C >= 221 and C(centre) <= 178
     proves C <= 220 for all nine pixels.  That brackets the median of the whole
     cell between two levels; four thresholds per cell then decide a pixel
     (defect / clean / ambiguous) and ambiguous pixels get an exact rank count.
-    Equals residual_mask_direct for ANY level set (tests/test_restate_vs_cv2.py)."""
+    Equals residual_mask_direct for ANY level set (tests/test_restate_vs_cv2.py).
+    `stats` receives lattice_stats' counts and pivot_counts, the exact window count of every list entry at its
+    own pivot."""
     levels = sorted(int(v) for v in levels)
-    K = len(levels)
     h, w = gray.shape
     g = gray.astype(np.int32)
-    ny, nx = (h + 2) // 3, (w + 2) // 3
-    # exact counts at virtual centres (3j+1, 3i+1): replicate padding also beyond the crop
-    pad = np.pad(gray, ((10, 10 + 3), (10, 10 + 3)), mode='edge')
-    cy = 3 * np.arange(ny) + 1
-    cx = 3 * np.arange(nx) + 1
-    lo_idx = np.zeros((ny, nx), np.int32)
-    n263 = np.zeros((ny, nx), np.int32)
-    for v in levels:
-        ind = (pad <= v).astype(np.int32)
-        s = np.pad(np.cumsum(np.cumsum(ind, axis=0), axis=1), ((1, 0), (1, 0)))
-        C = s[cy[:, None] + 21, cx[None, :] + 21] - s[cy[:, None], cx[None, :] + 21] \
-            - s[cy[:, None] + 21, cx[None, :]] + s[cy[:, None], cx[None, :]]
-        lo_idx += (C <= 178)
-        n263 += (C >= 263)
-    hi_idx = K - n263
-    LO = np.array([-1] + levels, np.int32)[lo_idx]
-    HI = np.array(levels + [255], np.int32)[hi_idx]
+    _, LO, HI = _lattice_brackets(gray, thr, levels)
     LOp = np.repeat(np.repeat(LO, 3, axis=0), 3, axis=1)[:h, :w]
     HIp = np.repeat(np.repeat(HI, 3, axis=0), 3, axis=1)[:h, :w]
     sure = (g <= LOp - thr) | (g >= HIp + thr + 1)
@@ -444,14 +488,39 @@ def residual_mask_lattice(gray, thr: int, levels, roi=None, stats: Optional[dict
     if roi is not None:
         amb &= roi
     out = sure.copy()
+    p10 = np.pad(gray, 10, mode='edge')
+    st = lattice_stats(gray, thr, levels, roi, cell_gray) if stats is not None else None
+    piv = []
+    for y, x in zip(*np.nonzero(amb)):
+        win = p10[y:y + 21, x:x + 21]
+        ca, cb = int((win <= g[y, x] + thr).sum()), int((win <= g[y, x] - thr - 1).sum())
+        out[y, x] = ca <= 220 or cb >= 221
+        if st is not None:
+            piv += ([ca] if st['ta'][y, x] else []) + ([cb] if st['tb'][y, x] else [])
     if stats is not None:
-        stats['ambiguous'] = int(amb.sum())
-    if amb.any():
-        p10 = np.pad(gray, 10, mode='edge')
-        for y, x in zip(*np.nonzero(amb)):
-            win = p10[y:y + 21, x:x + 21]
-            out[y, x] = int((win <= g[y, x] + thr).sum()) <= 220 or int((win <= g[y, x] - thr - 1).sum()) >= 221
+        stats.update({k: v for k, v in st.items() if k not in ('amb', 'ta', 'tb')})
+        stats['pivot_counts'] = np.array(piv, np.int32)
     return out
+
+
+def select_levels(hist, t_apx: int, thr: int, bright: bool = False):
+    """The median stage's three levels (csrc/vi_unit.cuh:99-137, select_levels): the lower median m of one
+    Otsu class of `hist` split at t_apx (the dark class g <= t_apx, or the bright one), then
+    [m - s, m, m + s] clamped to 0..254, s the largest power of two <= max(thr // 3, 1), at most 16.
+    An empty class takes m = t_apx."""
+    hist = np.asarray(hist, np.int64)
+    cum = np.cumsum(hist)
+    npix = int(cum[-1])
+    nd = int(cum[t_apx])
+    nb = npix - nd
+    ncls = nb if bright else nd
+    tgt = nd + (nb + 1) // 2 if bright else (nd + 1) // 2
+    m = int(np.argmax(cum >= tgt)) if ncls else int(t_apx)
+    s = 1
+    lim = max(thr // 3, 1)
+    while s * 2 <= lim and s < 16:
+        s *= 2
+    return [min(254, max(0, m - s)), min(254, max(0, m)), min(254, max(0, m + s))]
 
 
 # --------------------------------------------------------------------------- K14/K15

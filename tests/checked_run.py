@@ -68,6 +68,19 @@ def main():
     dn = torch.from_numpy(npix.astype(np.int32)).cuda()
     assert insp._lib.vi_debug_otsu(insp._ctx, dh.data_ptr(), dn.data_ptr(), len(H), out.data_ptr()) == _lib.VI_ERR_ARG
     torch.cuda.synchronize()
+    # the median residual stage on its own with its lists capped (every overflow path), and a batch of noisy plates
+    # whose units list from a few to more than 16,384 ambiguous pixels and more than 4,096 dirty cells
+    import test_gpu_median_residual as M
+    for (h, w) in ((315, 316), (48, 97), (24, 1500), (1, 4096)):
+        g = rng.integers(0, 256, size=(h, w), dtype=np.uint8)
+        roi = rng.random((h, w)) < 0.7
+        for ccap, ecap in ((4096, 16384), (0, 0), (1, 193), (7, 1), (4096, 192)):
+            _lib.check(M.stage(insp, g, roi, [100, 128, 156], 3, ccap, ecap)[0])
+    boxes, _, bottom = shelf_layout([(w, h, ph) for w, h, _, ph in M.UNITS], 1008)
+    fr = M.noisy_frames(boxes, [s for _, _, s, _ in M.UNITS], 3, bottom + 8, 1024, 500)
+    insp.configure(Grid(boxes=boxes), is_reference=True)
+    insp.inspect_batch(torch.from_numpy(fr).cuda(), vi_b200.default_params(threshold=6))
+    torch.cuda.synchronize()
     word = C.c_uint32(12345)
     _lib.check(insp._lib.vi_debug_check_word(insp._ctx, C.byref(word)))
     print("check_word", int(word.value))

@@ -46,7 +46,7 @@ EXPORTS = [
     "vi_packed_mask_offsets", "vi_host_upload_bytes", "vi_peer_table_create", "vi_peer_table_open", "vi_peer_table_close",
     "vi_peer_table_destroy", "vi_peer_table_read", "vi_set_record_peers", "vi_segment_cell", "vi_fill_internal_holes", "vi_mask_stats", "vi_erode_square",
     "vi_label_components", "vi_detect_defects", "vi_ingest_argb32", "vi_ingest_gray16", "vi_set_seg_stats_output", "vi_debug_set_profile", "vi_debug_check_word", "vi_debug_fastdiv_check", "vi_debug_otsu",
-    "vi_debug_adaptive_taps",
+    "vi_debug_rank_residual", "vi_debug_adaptive_taps",
 ]
 
 _lib = None
@@ -111,6 +111,8 @@ def load():
     lib.vi_debug_check_word.argtypes = [vp, P(C.c_uint32)]
     lib.vi_debug_fastdiv_check.argtypes = [vp, i64, C.c_uint64, P(i64)]
     lib.vi_debug_otsu.argtypes = [vp, vp, vp, C.c_int, vp]
+    lib.vi_debug_rank_residual.argtypes = [vp, vp, vp, C.c_int, C.c_int, P(C.c_int), C.c_int, C.c_int, C.c_int, C.c_int, vp,
+                                           P(C.c_int)]
     lib.vi_detect_defects.argtypes = [vp, vp, vp, C.c_int, C.c_int, P(ViParams), vp, P(i32), vp]
     lib.vi_debug_adaptive_taps.argtypes = [C.c_int, vp]
     lib.vi_set_seg_stats_output.argtypes = [vp, vp]

@@ -387,6 +387,84 @@ extern "C" int vi_debug_otsu(vi_ctx* c, const uint32_t* d_hists, const int* d_np
     return VI_OK;
 }
 
+// Diagnostics: the median residual stage on its own, one CTA running the device functions of the inspection kernel in
+// its order (vi_unit.cuh, P2 and P11): the crop's histogram and otsu_approx_warp on warp 0 next to the cell min / max
+// (the exact Otsu scan aside on kOtsuWarp when the V pass leaves it free), rank_cells, rank_finish.  The workspace is a
+// global arena as in the GMEM kernel; the crop is copied to the kernel's row pitch with `pad` in the bytes past w.
+// out[0] = ambiguous-pixel list entries (counters[1]), out[1] = dirty cells that touch the ROI (counters[0]), out[2] = otsu_t.
+__global__ void __launch_bounds__(kThreads) rank_debug_kernel(const uint8_t* src, const uint8_t* roi, Geom g, int3 lev, int thr,
+                                                              int ccap, int ecap, int pad, uint8_t* gray, unsigned* ROI,
+                                                              unsigned char* ws, unsigned char* lists, unsigned* clist,
+                                                              unsigned* elist, unsigned* CAND, int* out) {
+    __shared__ unsigned hist[256];
+    __shared__ __align__(16) double ows[kOtsuWsBytes / 8];
+    __shared__ int lv[kLevels], counters[4], otsu_last, otsu_t;
+    const int tid = threadIdx.x, npix = g.w * g.h;
+    for (int i = tid; i < g.h * g.gp; i += kThreads) {
+        const int y = i / g.gp, x = i - y * g.gp;
+        gray[i] = x < g.w ? src[y * g.w + x] : (uint8_t)pad;
+    }
+    for (int i = tid; i < g.nwords; i += kThreads) CAND[i] = 0;
+    if (tid < 256) hist[tid] = 0;
+    if (tid == 0) { lv[0] = lev.x; lv[1] = lev.y; lv[2] = lev.z; otsu_last = -1; }
+    load_mask_bits(roi, g, ROI);
+    cta_sync();
+    for (int i = tid; i < npix; i += kThreads) atomicAdd(&hist[src[i]], 1u);
+    cta_sync();
+    RankWs rw = rank_ws_carve(ws, g, lists, g.w, g.h, counters);
+    const bool oside = rank_otsu_aside(g);
+    PhaseTimerT<false> pt;
+    if (warp_id() == 0) {
+        int last;
+        otsu_approx_warp(hist, npix, last);
+        if (lane_id() == 0) *const_cast<volatile int*>(&otsu_last) = last;
+        rank_tables(lv, thr, rw);
+    } else if (oside && warp_id() == kOtsuWarp) {
+        const int t = otsu_scan(hist, npix, ows, &otsu_last, pt);
+        if (lane_id() == 0) otsu_t = t;
+    } else {
+        rank_cmm(gray, g, rw, 1, oside ? kWarps - 1 : kWarps, 0, rank_cmm_split(g, oside));
+    }
+    if (oside) { if (warp_id() != kOtsuWarp) workers_sync(kThreads - 32); } else cta_sync();
+    rank_cells(gray, g, rw, lv, hist, npix, ows, &otsu_last, &otsu_t, oside, pt);
+    rank_finish(gray, g, rw, lv, thr, ROI, CAND, clist, ccap, elist, ecap, pt);
+    if (tid == 0) { out[0] = counters[1]; out[1] = counters[0]; out[2] = otsu_t; }
+}
+
+extern "C" int vi_debug_rank_residual(vi_ctx* c, const uint8_t* d_gray, const uint8_t* d_roi, int w, int h, const int* levels,
+                                      int thr, int ccap, int ecap, int pad, uint32_t* d_cand, int* counts) {
+    if (!c || !d_gray || !d_roi || !levels || !d_cand || !counts) return fail(VI_ERR_ARG, "vi_debug_rank_residual: null");
+    if (w < 1 || h < 1 || w > kMaxUnitW || h > kMaxUnitH || (long long)w * h > kMaxUnitPixels)
+        return fail(VI_ERR_ARG, "vi_debug_rank_residual: %dx%d is outside the unit bound", w, h);
+    if (levels[0] < 0 || levels[0] > levels[1] || levels[1] > levels[2] || levels[2] > 255)
+        return fail(VI_ERR_ARG, "vi_debug_rank_residual: levels must be sorted and in 0..255");
+    if (thr < 0 || thr > 255 || pad < 0 || pad > 255) return fail(VI_ERR_ARG, "vi_debug_rank_residual: thr and pad must be in 0..255");
+    if (ccap < 0 || ccap > kDirtyListCap || ecap < 0 || ecap > kExactListCap)
+        return fail(VI_ERR_ARG, "vi_debug_rank_residual: ccap in 0..%d, ecap in 0..%d", kDirtyListCap, kExactListCap);
+    VI_DEVICE(c);
+    const Geom g = make_geom(w, h);
+    const long long gray_b = ((long long)g.gp * h + 255) & ~255ll, roi_b = ((long long)g.nwords * 4 + 255) & ~255ll;
+    const long long ws_b = (rank_ws_bytes(w, h) + 255) & ~255ll, plane_b = (rank_plane_words(w, h) * 4 + 255) & ~255ll;
+    const long long total = gray_b + roi_b + ws_b + plane_b + 4ll * (kDirtyListCap + kExactListCap) + 16;
+    unsigned char* d = nullptr;
+    CU(cudaMalloc(&d, total));
+    unsigned char* p = d;
+    uint8_t* gray = p; p += gray_b;
+    unsigned* roi = reinterpret_cast<unsigned*>(p); p += roi_b;
+    unsigned char* ws = p; p += ws_b;
+    unsigned char* lists = p; p += plane_b;
+    unsigned* clist = reinterpret_cast<unsigned*>(p); p += 4ll * kDirtyListCap;
+    unsigned* elist = reinterpret_cast<unsigned*>(p); p += 4ll * kExactListCap;
+    int* d_out = reinterpret_cast<int*>(p);
+    rank_debug_kernel<<<1, kThreads>>>(d_gray, d_roi, g, make_int3(levels[0], levels[1], levels[2]), thr, ccap, ecap, pad, gray, roi,
+                                       ws, lists, clist, elist, d_cand, d_out);
+    cudaError_t e = cudaGetLastError();
+    if (e == cudaSuccess) e = cudaMemcpy(counts, d_out, 3 * sizeof(int), cudaMemcpyDeviceToHost);
+    cudaFree(d);
+    if (e != cudaSuccess) return fail(VI_ERR_CUDA, "vi_debug_rank_residual: %s", cudaGetErrorString(e));
+    return VI_OK;
+}
+
 extern "C" int vi_debug_check_word(vi_ctx* c, uint32_t* out) {
     if (!c || !out) return fail(VI_ERR_ARG, "vi_debug_check_word: null");
 #ifdef VI_CHECKED

@@ -64,6 +64,7 @@ struct RankWs {
 
 constexpr int kExactCap = 4096;
 constexpr int kExactWarpMax = 192;       // more ambiguous pixels than this: one thread per pixel instead of one warp
+constexpr int kDirtyListCap = 4096, kExactListCap = 16384;     // rank_finish's lists in the labelling workspace hold at most these
 __host__ __device__ inline long long rank_plane_words(int wmax, int hmax) {
     return (long long)rank_ngrp(wmax) * ((((hmax + kCell - 1) / kCell) + 15) & ~15);
 }

@@ -558,7 +558,7 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
     if (SPEC || lattice) {
         RankWs rw = rank_ws_carve(Rg + plan.mask_bytes, g, g_rank, a.wmax, a.hmax, sh.rank_cnt);
         // lists of the stage in the (free) labelling workspace: dirty cells of the ROI, ambiguous pixels
-        const int ccap = min(plan.ws_bytes >> 4, 4096), ecap = min((plan.ws_bytes >> 2) - ccap, 16384);
+        const int ccap = min(plan.ws_bytes >> 4, kDirtyListCap), ecap = min((plan.ws_bytes >> 2) - ccap, kExactListCap);
         n_amb = rank_finish(gray, g, rw, sh.levels, thr, MD, CAND, reinterpret_cast<unsigned*>(WS), ccap,
                             reinterpret_cast<unsigned*>(WS) + ccap, ecap, pt);
         if (SPEC) {
