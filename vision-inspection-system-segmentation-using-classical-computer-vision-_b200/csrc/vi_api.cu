@@ -69,12 +69,10 @@ struct GridState {
     std::vector<int4> rects;
     std::vector<long long> off;     // n+1
     long long unit_px = 0;
-    int wmax = 0, hmax = 0;
+    UnitExtent ext{};               // the largest unit: sizes the kernel's layout (unit_layout)
     std::vector<long long> woff;    // n+1: packed-bit mask offsets in 32-bit words
     long long unit_words = 0;
     DevBuf d_rects, d_off, d_woff;
-    SmemPlan plan{};
-    bool gmem = false;              // units beyond one SM's shared memory: the global-arena kernel
 };
 
 struct vi_ctx {
@@ -91,10 +89,6 @@ struct vi_ctx {
     int is_reference = 0;
     DevBuf scratch;
     DevBuf arena;
-    long long scratch_stride = 0;
-    long long scratch_f32_off = 0;
-    long long scratch_rank_off = 0;
-    long long scratch_blob_off = 0;
     // compat / host-batch staging
     DevBuf st_in, st_aux, st_out, st_out2, st_rec, st_stats, st_lab;
     DevBuf hb_frames[kHostSlots], hb_seg[kHostSlots], hb_def[kHostSlots], hb_rec[kHostSlots], hb_blob[kHostSlots];
@@ -202,7 +196,7 @@ static int set_grid_state(vi_ctx* c, GridState& gs, const int32_t* r, int n, cud
     gs.rects.resize(n);
     gs.off.assign(n + 1, 0);
     gs.woff.assign(n + 1, 0);
-    gs.wmax = gs.hmax = 0;
+    gs.ext = UnitExtent{};
     for (int i = 0; i < n; ++i) {
         int x = r[4 * i], y = r[4 * i + 1], w = r[4 * i + 2], h = r[4 * i + 3];
         if (w <= 0 || h <= 0 || x < 0 || y < 0) return fail(VI_ERR_ARG, "grid: rect %d = (%d,%d,%d,%d) is invalid", i, x, y, w, h);
@@ -212,27 +206,17 @@ static int set_grid_state(vi_ctx* c, GridState& gs, const int32_t* r, int n, cud
         gs.rects[i] = make_int4(x, y, w, h);
         gs.off[i + 1] = gs.off[i] + (long long)w * h;
         gs.woff[i + 1] = gs.woff[i] + (long long)((w + 31) / 32) * h;
-        gs.wmax = std::max(gs.wmax, w);
-        gs.hmax = std::max(gs.hmax, h);
+        gs.ext.add(w, h);
     }
     gs.unit_px = gs.off[n];
     gs.unit_words = gs.woff[n];
-    int gray_need = 0, words_need = 0;
-    for (int i = 0; i < n; ++i) {
-        const Geom g = make_geom(gs.rects[i].z, gs.rects[i].w);
-        gray_need = std::max(gray_need, g.gp * g.h);
-        words_need = std::max(words_need, g.nwords);
-    }
-    gs.gmem = false;
-    if (!make_plan(gs.wmax, gs.hmax, c->smem_optin, c->smem_static, &gs.plan, gray_need, words_need)) {
-        // larger than one SM's shared memory: same pipeline over a per-CTA arena in global memory.  The pixel bound
-        // holds per unit (checked above); a ragged grid's wmax x hmax may exceed it (a 4096 x 200 strip next to a
-        // 200 x 8000 column), and everything sized from wmax x hmax is 64-bit or within int range up to 4096 x 8192.
-        gs.gmem = true;
-        if (!make_plan_gmem(gs.wmax, gs.hmax, &gs.plan, gray_need, words_need))
-            return fail(VI_ERR_TOO_LARGE, "grid: units up to %d x %d exceed the bound of a unit (%d wide, %d high)",
-                        gs.wmax, gs.hmax, kMaxUnitW, kMaxUnitH);
-    }
+    // Units larger than one SM's shared memory take the arena kernel.  The pixel bound holds per unit (checked above);
+    // a ragged grid's wmax x hmax may exceed it (a 4096 x 200 strip next to a 200 x 8000 column), and everything sized
+    // from wmax x hmax is 64-bit or within int range up to 4096 x 8192.
+    UnitLayout layout;
+    if (!unit_layout(gs.ext, c->smem_optin, c->smem_static, false, 0, &layout))
+        return fail(VI_ERR_TOO_LARGE, "grid: units up to %d x %d exceed the bound of a unit (%d wide, %d high)",
+                    gs.ext.wmax, gs.ext.hmax, kMaxUnitW, kMaxUnitH);
     int rc;
     if ((rc = gs.d_rects.ensure(sizeof(int4) * n))) return rc;
     if ((rc = gs.d_off.ensure(sizeof(long long) * (n + 1)))) return rc;
@@ -411,7 +395,7 @@ __global__ void __launch_bounds__(kThreads) rank_debug_kernel(const uint8_t* src
     cta_sync();
     for (int i = tid; i < npix; i += kThreads) atomicAdd(&hist[src[i]], 1u);
     cta_sync();
-    RankWs rw = rank_ws_carve(ws, g, lists, g.w, g.h, counters);
+    RankWs rw = rank_ws_carve(ws, g, lists, (int)rank_plane_words(g.w, g.h), counters);
     const bool oside = rank_otsu_aside(g);
     PhaseTimerT<false> pt;
     if (warp_id() == 0) {
@@ -713,22 +697,6 @@ static int fill_params(KArgs& a, const vi_params* p) {
     return VI_OK;
 }
 
-static long long scratch_layout(vi_ctx* c, int wmax, int hmax, bool f32_plane, int blob_k) {
-    long long px = (long long)wmax * hmax;
-    long long capg = (long long)hmax * (wmax / 2 + 1);
-    long long px4 = (long long)((wmax + 3) & ~3) * hmax;
-    long long stride = ((px * 2 + 15) & ~15ll) + ((px4 + 15) & ~15ll) + (long long)ccl_ws_bytes((int)capg, hmax) + 256;
-    stride = (stride + 255) & ~255ll;
-    c->scratch_rank_off = stride;
-    stride += (rank_scratch_bytes(wmax, hmax) + 255) & ~255ll;
-    c->scratch_f32_off = stride;
-    if (f32_plane) stride += (px * 4 + 255) & ~255ll;       // float plane of the adaptive mean, only when asked for
-    c->scratch_blob_off = stride;
-    stride += ((long long)blob_k * sizeof(BlobAcc) + 255) & ~255ll;   // blob accumulators that do not fit two masks
-    c->scratch_stride = stride;
-    return stride;
-}
-
 // The frames as a tensor map for the kernel's asynchronous crop gather (vi_pipeline.cuh: gather_issue_tma).  The
 // encoder is a driver entry point; it is looked up through the runtime so the library keeps linking against cudart
 // only.  Returns false (a.tma_ok = 0: the kernel falls back to one bulk copy per crop row) when anything does not fit.
@@ -756,15 +724,15 @@ static bool make_frame_tensor(KArgs& a, const GridState& gs) {
     if (!enc) return false;
     // the aligned span of a crop: up to 15 bytes of phase in front; tiles of equal width (a multiple of 16) and whole
     // boxes of rows (a multiple of 8 high: every box starts 128-byte aligned); the fewest column boxes that fit the staging area
-    const int w16 = (gs.wmax + 15 + 15) & ~15;
-    const int nrb = (gs.hmax + 255) / 256;
-    const int bh = (((gs.hmax + nrb - 1) / nrb) + 7) & ~7;
+    const int w16 = (gs.ext.wmax + 15 + 15) & ~15;
+    const int nrb = (gs.ext.hmax + 255) / 256;
+    const int bh = (((gs.ext.hmax + nrb - 1) / nrb) + 7) & ~7;
     if (bh > 256) return false;
     int ncb = 0, bw = 0, tile_bytes = 0;
     for (int n = (w16 + 255) / 256; n <= 4; ++n) {
         const int b = (((w16 + n - 1) / n) + 15) & ~15;
         const int t = (b * bh * nrb + 127) & ~127;
-        if (b <= 256 && (long long)n * t <= (long long)gs.plan.gray_bytes + gs.plan.mask_bytes) { ncb = n; bw = b; tile_bytes = t; break; }
+        if (b <= 256 && (long long)n * t <= a.layout.stage_bytes) { ncb = n; bw = b; tile_bytes = t; break; }
     }
     if (!ncb) return false;
     if ((a.row_pitch & 15) || (a.n_images > 1 && (a.image_stride & 15)) || (reinterpret_cast<uintptr_t>(a.frames) & 15)) return false;
@@ -790,25 +758,19 @@ static int launch_units(vi_ctx* c, KArgs& a, const GridState& gs, cudaStream_t s
     if (n_total <= 0) return VI_OK;
     if (n_total > 0x7fffffffll) return fail(VI_ERR_ARG, "too many units in one call");
     int rc;
-    const long long stride = scratch_layout(c, gs.wmax, gs.hmax, a.p.seg_method == 1, a.blobs ? a.blob_k : 0);
-    const long long astride = gs.gmem ? plan_arena_bytes(gs.plan) : 0;
+    UnitLayout& L = a.layout;
+    unit_layout(gs.ext, c->smem_optin, c->smem_static, a.p.seg_method == 1, a.blobs ? a.blob_k : 0, &L);   // (checked by set_grid_state)
+    const long long stride = L.scratch_bytes, astride = L.arena_bytes;
     // CTAs per slot: one per SM; fewer when the units are so large that their scratch would not fit the budget
     int bps = c->sm_count;
     if ((stride + astride) * kHostSlots * bps > kScratchBudget)
         bps = (int)std::max<long long>(1, kScratchBudget / ((stride + astride) * kHostSlots));
     const int nblocks = (int)std::min<long long>(n_total, bps);
     if ((rc = c->scratch.ensure((size_t)stride * kHostSlots * bps))) return rc;
-    if (gs.gmem && (rc = c->arena.ensure((size_t)astride * kHostSlots * bps))) return rc;
+    if (L.arena && (rc = c->arena.ensure((size_t)astride * kHostSlots * bps))) return rc;
     a.scratch = (uint8_t*)c->scratch.p + (size_t)slot * bps * stride;
-    a.scratch_stride = stride;
-    a.scratch_f32_off = c->scratch_f32_off;
-    a.scratch_rank_off = c->scratch_rank_off;
-    a.scratch_blob_off = c->scratch_blob_off;
-    a.arena = gs.gmem ? (uint8_t*)c->arena.p + (size_t)slot * bps * astride : nullptr;
-    a.arena_stride = astride;
-    a.wmax = gs.wmax; a.hmax = gs.hmax;
-    a.plan = gs.plan;
-    if (c->smem_set < gs.plan.total) {
+    a.arena = L.arena ? (uint8_t*)c->arena.p + (size_t)slot * bps * astride : nullptr;
+    if (c->smem_set < L.total) {
         const int lim = c->smem_optin - c->smem_static;
         CU(cudaFuncSetAttribute(vi_unit_kernel<false, false, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
         CU(cudaFuncSetAttribute(vi_unit_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
@@ -818,11 +780,11 @@ static int launch_units(vi_ctx* c, KArgs& a, const GridState& gs, cudaStream_t s
         CU(cudaFuncSetAttribute(vi_unit_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
         c->smem_set = lim;
     }
-    if (gs.plan.total > c->smem_set) return fail(VI_ERR_TOO_LARGE, "shared-memory plan %d > %d", gs.plan.total, c->smem_set);
-    if (gs.gmem) {
+    if (L.total > c->smem_set) return fail(VI_ERR_TOO_LARGE, "shared-memory plan %d > %d", L.total, c->smem_set);
+    if (L.arena) {
         // units beyond one SM's shared memory (DESIGN.md section 2): same phases over the CTA's global arena
         a.prof = nullptr;
-        vi_unit_kernel<false, false, true><<<nblocks, kThreads, gs.plan.total, stream>>>(a);
+        vi_unit_kernel<false, false, true><<<nblocks, kThreads, L.total, stream>>>(a);
         CU(cudaGetLastError());
         return VI_OK;
     }
@@ -830,14 +792,14 @@ static int launch_units(vi_ctx* c, KArgs& a, const GridState& gs, cudaStream_t s
     bool spec = a.mode == MODE_FULL && a.blur_k == 3 && a.se_k == 3 && a.p.seg_method == 0 && a.p.defect_method == 0 &&
                 !a.labels_out && !a.seg_stats && !a.seg_bits && !a.def_bits && !a.aux_mask && !a.stats_out &&
                 (a.row_pitch & 15) == 0 && (reinterpret_cast<uintptr_t>(a.frames) & 15) == 0 && (a.image_stride & 15) == 0 &&
-                rank_ws_bytes(gs.wmax, gs.hmax) + kOtsuWsBytes <= (long long)(kNumMasks - 1) * gs.plan.mask_bytes + gs.plan.ws_bytes && gs.plan.n_hist >= kWarps / 2;
+                lattice_fits(gs.ext.wmax, gs.ext.hmax, L) && hist_round_fits(L.n_hist);
     if (spec) make_frame_tensor(a, gs);
 #ifndef VI_CHECKED
-    if (a.prof && spec) vi_unit_kernel<true, true, false><<<nblocks, kThreads, gs.plan.total, stream>>>(a);   // diagnostics build: phase timers
+    if (a.prof && spec) vi_unit_kernel<true, true, false><<<nblocks, kThreads, L.total, stream>>>(a);   // diagnostics build: phase timers
     else
 #endif
-    if (spec) vi_unit_kernel<false, true, false><<<nblocks, kThreads, gs.plan.total, stream>>>(a);
-    else { a.prof = nullptr; vi_unit_kernel<false, false, false><<<nblocks, kThreads, gs.plan.total, stream>>>(a); }
+    if (spec) vi_unit_kernel<false, true, false><<<nblocks, kThreads, L.total, stream>>>(a);
+    else { a.prof = nullptr; vi_unit_kernel<false, false, false><<<nblocks, kThreads, L.total, stream>>>(a); }
     CU(cudaGetLastError());
     return VI_OK;
 }

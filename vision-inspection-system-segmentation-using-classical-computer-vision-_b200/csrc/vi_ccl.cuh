@@ -35,13 +35,10 @@ struct CclWs {
     __device__ __forceinline__ unsigned short* yy() const { return reinterpret_cast<unsigned short*>(base + rf + (cap + 1) * 16); }
 };
 
-__host__ __device__ inline size_t ccl_ws_bytes(int cap, int h) {
-    return (size_t)align16((h + 2) * 4) + (size_t)(cap + 1) * 18 + 64;
-}
-
-__device__ inline CclWs ccl_ws_carve(unsigned char* base, int cap, int h) {
+// A table of `cap` runs at `base` takes ccl_ws_bytes(cap, h) (vi_device.cuh); `rf` = ccl_rowfirst_bytes(h).
+__device__ inline CclWs ccl_ws_carve(unsigned char* base, int cap, int rf) {
     CclWs ws;
-    ws.base = base; ws.cap = cap; ws.rf = align16((h + 2) * 4);
+    ws.base = base; ws.cap = cap; ws.rf = rf;
     return ws;
 }
 
@@ -456,14 +453,6 @@ VI_PHASE void ccl_paint(unsigned* dst, const unsigned* base, const Geom& g, cons
         dst[i] = base ? (base[i] | bits) : bits;
     }
 }
-
-// Accumulator of one kept component of the defect-blob table (vi_set_defect_blob_output): pixel area, bounding box
-// and coordinate sums over its runs; ymin is the root run's row, area2 the area filter's acc0.
-struct BlobAcc {
-    unsigned long long sx, sy;
-    unsigned area, xmin, xmax, ymin, ymax, area2;
-};
-static_assert(sizeof(BlobAcc) == 40, "BlobAcc layout");
 
 // The first kc kept components of a labelling (after ccl_build and the per-root acc0 of the area filter), in raster
 // order of their first pixel, into out[0..kc).  acc1[root] = 1 + slot (an exclusive count of kept roots in increasing

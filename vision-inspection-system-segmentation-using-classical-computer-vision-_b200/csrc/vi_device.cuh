@@ -6,6 +6,7 @@
 // Reference semantics: SURVEY.md Appendix A; every stage cites the reference
 // call site it reproduces (paths under the reference tree).
 #pragma once
+#include <algorithm>
 #include <cstdint>
 #include <type_traits>
 #include <cuda.h>              // CUtensorMap (type only: the encoder is looked up through the runtime, no libcuda link)
@@ -93,7 +94,7 @@ __host__ __device__ inline Geom make_geom(int w, int h) {
     return g;
 }
 
-// Geometry of the median stage's lattice workspace (vi_rank.cuh), here because the plans below size it.
+// Geometry of the median stage's lattice workspace (vi_rank.cuh), here because the unit layout below sizes it.
 constexpr int kCell = 3;
 constexpr int kColsPerWarp = 30;         // V pass: 10 whole cells per warp
 constexpr int kVPad = 3;                 // virtual cells either side of a lattice row (the window is 7 cells wide)
@@ -116,88 +117,146 @@ __host__ __device__ inline long long rank_ws_bytes(int w, int h) {
     return ((((nly + 7) & ~7ll) + 1) * rank_P(w) * 4 + nly * rank_cpitch(w) * 2 + 64 + 15) & ~15ll;      // (+1: the row before row 0)
 }
 
+__host__ __device__ inline int align16(int v) { return (v + 15) & ~15; }
+__host__ __device__ inline long long align256(long long v) { return (v + 255) & ~255ll; }
 
-// Shared-memory plan for the largest unit of a grid (host computes, kernel follows).
-struct SmemPlan {
-    int gray_bytes;    // [0, gray_bytes): gray crop
-    int n_hist;        // lane-private histogram copies that fit next to the crop (1..16)
-    int mask_bytes;    // one bit-packed mask (16-B aligned)
-    int ws_bytes;      // workspace after the masks (run tables / Otsu arrays / rank-count band)
-    int run_cap;       // runs that fit the shared workspace
-    int band_pitch;    // uint2 entries per band row of the rank-count stage
-    int total;         // dynamic shared memory bytes
+// Sizes the unit layout below is built from, defined here and used by the phases that own the regions.
+constexpr int kOtsuWsBytes = 3 * 256 * (int)sizeof(double) + 64;     // exact Otsu scan arrays (vi_pipeline.cuh: otsu_scan)
+constexpr int kRunBytes = 18;                       // one run of a run table (vi_ccl.cuh: CclWs): parent, 2 accumulators, xs, xe, y
+__host__ __device__ inline int ccl_rowfirst_bytes(int h) { return align16((h + 2) * 4); }
+__host__ __device__ inline long long ccl_ws_bytes(long long cap, int h) { return ccl_rowfirst_bytes(h) + (cap + 1) * kRunBytes + 64; }
+__host__ __device__ inline int ccl_ws_cap(long long bytes, int h) { return (int)((bytes - ccl_rowfirst_bytes(h) - 64) / kRunBytes - 1); }
+// Rank plane of the median stage's cell pass (vi_rank.cuh: RankWs::plane) and its list of ambiguous pixels, in scratch.
+constexpr int kExactCap = 4096;
+__host__ __device__ inline long long rank_plane_words(int wmax, int hmax) { return (long long)rank_ngrp(wmax) * ((((hmax + kCell - 1) / kCell) + 15) & ~15); }
+__host__ __device__ inline long long rank_scratch_bytes(int wmax, int hmax) { return rank_plane_words(wmax, hmax) * 4 + kExactCap * 4; }
+constexpr int kDirtyListCap = 4096, kExactListCap = 16384;     // rank_finish's lists in the labelling workspace hold at most these
+// Accumulator of one kept component of the defect-blob table (vi_ccl.cuh: ccl_blob_table): pixel area, bounding box
+// and coordinate sums over its runs; ymin is the root run's row, area2 the area filter's acc0.
+struct BlobAcc {
+    unsigned long long sx, sy;
+    unsigned area, xmin, xmax, ymin, ymax, area2;
+};
+static_assert(sizeof(BlobAcc) == 40, "BlobAcc layout");
+
+// The largest unit of a grid: its width and height, and the largest crop (gray pitch x height) and bit mask over the
+// units (a ragged grid's widest and tallest units need not be the same one).
+struct UnitExtent {
+    int wmax, hmax, gray_need, mask_words;
+    __host__ void add(int w, int h) {
+        const Geom g = make_geom(w, h);
+        wmax = std::max(wmax, w); hmax = std::max(hmax, h);
+        gray_need = std::max(gray_need, g.gp * h); mask_words = std::max(mask_words, g.nwords);
+    }
 };
 
-__host__ __device__ inline int align16(int v) { return (v + 15) & ~15; }
+// Memory layout of one CTA of vi_unit_kernel, computed on the host per launch (unit_layout) and only read by the kernel.
+//
+// Dynamic shared memory -- in the arena kernel (GMEM) the CTA's arena in global memory, offsets the same -- holds the
+// gray crop, five bit-packed masks MA..ME and a workspace:
+//
+//   [ gray | MA | MB | MC | MD | ME | workspace ..................... Otsu ]
+//
+// Phases reuse regions that are dead at the time.  Alias table -- region: the phases that own it; what it overlaps:
+//   hist      blur + histogram (P1), shared-memory kernel only (the arena kernel keeps all 16 copies in shared memory
+//             and the rest in the arena): n_hist copies from MA on;  MA..ME, workspace and what lies in them
+//   lattice   the median stage's cell pass (P2, with the Otsu scan; the pass leaves its results in the scratch plane);
+//             MB..ME, workspace up to the Otsu arrays, and the lists and tables below that live there later
+//   otsu      the exact Otsu scan (P2);  workspace, run table, dirty / exact lists
+//   band      the inverse threshold's uncertain pixels (P3);  MD, ME, lattice, blob table
+//   runs      labelling (P5 hole fill to P14);  workspace, lattice, Otsu arrays, dirty / exact lists
+//   dirty     dirty cells of the ROI (P11, rank_finish), exact = ambiguous pixels after them;  workspace, lattice,
+//             Otsu arrays, run table (the ROI's labelling is done, the defects' has not started)
+//   blob      kept-component accumulators (P14);  MC, MD (dead after the area filter), lattice, band; when they do
+//             not fit, the scratch blob tail
+//   stage     the next unit's crop gather, from rank_finish (P11) on (shared-memory kernel);  gray, MA (the ROI pass
+//             is done with both)
+// Per-CTA scratch in global memory (scratch_bytes apart, L2-resident), no aliases:
+//   [ u16 hsum | u8 blurred (rows of whole words) | run-table overflow | rank plane + exact list | f32 plane | blobs ]
+struct UnitLayout {
+    int gray_bytes;             // gray crop at 0
+    int mask_bytes;             // mask k (MA..ME) at gray_bytes + k * mask_bytes; 16-byte multiple
+    int ws_off, ws_bytes;       // workspace after the masks
+    int otsu_off;               // the last kOtsuWsBytes of the workspace
+    int stage_bytes;            // staging area of the crop gather at 0 (128-byte aligned: the dynamic base is)
+    int lattice_off;            // the median stage's lattice, from MB on
+    int n_hist;                 // lane-private histogram copies that fit (1..16), from MA on (shared-memory kernel)
+    int run_rf;                 // row_first bytes of both run tables
+    int run_cap;                // runs of the table in the workspace
+    int band_off, band_cap;     // inverse threshold's uncertain-pixel list, in words
+    int dirty_cap, exact_cap;   // rank_finish's lists: dirty cells at ws_off, ambiguous pixels after them (words)
+    int blob_off, blob_cap;     // kept-component accumulators in the masks
+    int total;                  // dynamic shared memory bytes
+    int arena;                  // units beyond one SM's shared memory: the arena kernel
+    long long lattice_bytes;    // room for the lattice from lattice_off up to the Otsu arrays (lattice_fits)
+    long long arena_bytes;      // per-CTA arena (arena kernel)
+    // scratch, after the u16 horizontal sums at 0: blurred crop, run-table overflow (runs_cap runs), rank plane
+    // (rank_words) and kExactCap ambiguous pixels, float plane of the adaptive mean, blobs that do not fit the masks
+    long long blur_off, runs_off;
+    int runs_cap;
+    long long rank_off;
+    int rank_words;
+    long long f32_off, blob_tail_off, scratch_bytes;
+};
 
-// gray_need / mask_words_need: the largest crop and the largest bit mask over the grid's units (a ragged grid's widest
-// and tallest units need not be the same one); 0 = take them from a wmax x hmax unit.
-__host__ inline bool make_plan(int wmax, int hmax, int smem_limit, int fixed, SmemPlan* p, int gray_need = 0, int mask_words_need = 0) {
-    Geom g = make_geom(wmax, hmax);
-    p->gray_bytes = align16(gray_need > 0 ? gray_need : g.gp * hmax);
-    p->mask_bytes = align16((mask_words_need > 0 ? mask_words_need : g.nwords) * 4);
-    p->band_pitch = 0;
-    int otsu = 3 * 256 * 8 + 64;                // vi_pipeline.cuh: kOtsuWsBytes, at the end of the workspace
-    int band = otsu;                            // (the median stage's lattice lives in the mask region: no claim here)
-    int rowfirst = align16((hmax + 2) * 4);
-    int want_cap = 2048;
-    int ccl = rowfirst + (want_cap + 1) * 18 + 64;
-    int ws = band > otsu ? band : otsu;
-    if (ccl > ws) ws = ccl;
-    ws = align16(ws);
-    // `fixed`: the kernel's static shared memory (CTA histogram, scan scratch, scalars)
-    int avail = smem_limit - fixed - p->gray_bytes;
-    int need_r = kNumMasks * p->mask_bytes + ws;
-    if (avail < need_r || avail < kHistBytes) return false;
-    int nh = avail / kHistBytes;
-    if (nh > kWarps) nh = kWarps;
-    p->n_hist = nh;
-    int r_bytes = nh * kHistBytes;
-    if (r_bytes < need_r) r_bytes = need_r;
-    // spend what is left of the hist region on a larger run table
-    int spare = r_bytes - kNumMasks * p->mask_bytes;
-    if (spare > ws) ws = spare & ~15;
-    p->ws_bytes = ws;
-    p->run_cap = (ws - rowfirst - 64) / 18 - 1;
-    if (p->run_cap > 65534) p->run_cap = 65534;
-    p->total = p->gray_bytes + r_bytes;
-    return true;
-}
+// The median stage's lattice of a w x h unit fits the layout.
+__host__ __device__ inline bool lattice_fits(int w, int h, const UnitLayout& L) { return rank_ws_bytes(w, h) <= L.lattice_bytes; }
+// Enough histogram copies for one round of blur3_hist.
+__host__ __device__ inline bool hist_round_fits(int n_hist) { return n_hist >= kWarps / 2; }
 
-// Plan for units that do not fit one SM's shared memory: the same regions, laid out in a per-CTA arena in global memory
-// (L2-resident for mid-size units); only the lane-private histogram copies stay in shared memory.  `total` is the
-// dynamic shared memory (the histogram copies), the arena needs gray_bytes + kNumMasks * mask_bytes + ws_bytes.
 // Bounds of a unit: 255 * pixels must fit 32 bits (histogram moments), and the index arithmetic of the phases
 // (magic_div: n * d < 2^32) holds for w <= 4096, h <= 8192.  A whole 4096x3000 frame is a legal unit.  The pixel bound
 // is a bound per unit (vi_api.cu: set_grid_state): a ragged grid's largest width and largest height, which size the
-// plan and the per-CTA scratch, may come from different units and multiply to more than 2^24.
+// layout and the per-CTA scratch, may come from different units and multiply to more than 2^24.
 constexpr long long kMaxUnitPixels = 1ll << 24;
 constexpr int kMaxUnitW = 4096, kMaxUnitH = 8192;
 
-__host__ inline bool make_plan_gmem(int wmax, int hmax, SmemPlan* p, int gray_need, int mask_words_need) {
-    if (wmax > kMaxUnitW || hmax > kMaxUnitH) return false;
-    Geom g = make_geom(wmax, hmax);
-    p->gray_bytes = align16(gray_need > 0 ? gray_need : g.gp * hmax);
-    p->mask_bytes = align16((mask_words_need > 0 ? mask_words_need : g.nwords) * 4);
-    p->band_pitch = 0;
-    int otsu = 3 * 256 * 8 + 64;
-    int rowfirst = align16((hmax + 2) * 4);
-    int want_cap = 8192;
-    int ccl = rowfirst + (want_cap + 1) * 18 + 64;
-    // the median stage's lattice (vi_rank.cuh) spans the masks after the first and this workspace
-    long long rank = rank_ws_bytes(wmax, hmax) + otsu - (long long)(kNumMasks - 1) * p->mask_bytes;
-    long long ws = rank > ccl ? rank : ccl;
-    if (ws > 0x7fff0000ll) return false;
-    p->ws_bytes = align16((int)ws);
-    p->run_cap = (p->ws_bytes - rowfirst - 64) / 18 - 1;
-    if (p->run_cap > 65534) p->run_cap = 65534;
-    p->n_hist = kWarps;
-    p->total = kWarps * kHistBytes;
+// The layout for units up to `e`, the device's opt-in shared memory and the kernel's static shared memory (CTA
+// histogram, scan scratch, scalars), and the call's options: the adaptive mean's float plane, `blob_k` kept components.
+// Shared memory when everything fits one SM (the histogram copies take what is left, the run table what they leave
+// past the masks), else the arena in global memory with all 16 histogram copies in shared memory.  False: beyond the
+// bound of a unit.
+__host__ inline bool unit_layout(const UnitExtent& e, int smem_optin, int smem_static, bool f32_plane, int blob_k, UnitLayout* out) {
+    UnitLayout L{};
+    L.gray_bytes = align16(e.gray_need);
+    L.mask_bytes = align16(e.mask_words * 4);
+    const int masks = kNumMasks * L.mask_bytes;
+    const int avail = smem_optin - smem_static - L.gray_bytes;
+    int ws = align16(std::max<long long>(kOtsuWsBytes, ccl_ws_bytes(2048, e.hmax)));
+    if (avail >= masks + ws && avail >= kHistBytes) {
+        L.n_hist = std::min(avail / kHistBytes, kWarps);
+        const int r_bytes = std::max(L.n_hist * kHistBytes, masks + ws);
+        if (r_bytes - masks > ws) ws = (r_bytes - masks) & ~15;
+        L.total = L.gray_bytes + r_bytes;
+    } else {
+        if (e.wmax > kMaxUnitW || e.hmax > kMaxUnitH) return false;
+        // the median stage's lattice at wmax x hmax spans the masks after the first and this workspace
+        const long long lat = rank_ws_bytes(e.wmax, e.hmax) + kOtsuWsBytes - (long long)(kNumMasks - 1) * L.mask_bytes;
+        const long long w = std::max(lat, ccl_ws_bytes(8192, e.hmax));
+        if (w > 0x7fff0000ll) return false;
+        ws = align16((int)w);
+        L.n_hist = kWarps; L.total = kWarps * kHistBytes;
+        L.arena = 1; L.arena_bytes = align256((long long)L.gray_bytes + masks + ws);
+    }
+    L.ws_off = L.gray_bytes + masks; L.ws_bytes = ws;
+    L.otsu_off = L.ws_off + ws - kOtsuWsBytes;
+    L.stage_bytes = L.lattice_off = L.gray_bytes + L.mask_bytes;
+    L.lattice_bytes = (long long)L.otsu_off - L.lattice_off;
+    L.run_rf = ccl_rowfirst_bytes(e.hmax); L.run_cap = std::min(ccl_ws_cap(ws, e.hmax), 65534);
+    L.band_off = L.gray_bytes + 3 * L.mask_bytes; L.band_cap = 2 * (L.mask_bytes / 4);
+    L.dirty_cap = std::min(ws >> 4, kDirtyListCap); L.exact_cap = std::min((ws >> 2) - L.dirty_cap, kExactListCap);
+    L.blob_off = L.gray_bytes + 2 * L.mask_bytes; L.blob_cap = 2 * L.mask_bytes / (int)sizeof(BlobAcc);
+    const long long px = (long long)e.wmax * e.hmax;
+    L.blur_off = (px * 2 + 15) & ~15ll;
+    L.runs_off = L.blur_off + (((long long)((e.wmax + 3) & ~3) * e.hmax + 15) & ~15ll);     // blurred rows: whole words
+    L.runs_cap = e.hmax * (e.wmax / 2 + 1);
+    L.rank_off = align256(L.runs_off + ccl_ws_bytes(L.runs_cap, e.hmax) + 256);
+    L.rank_words = (int)rank_plane_words(e.wmax, e.hmax);
+    L.f32_off = L.rank_off + align256(rank_scratch_bytes(e.wmax, e.hmax));
+    L.blob_tail_off = L.f32_off + (f32_plane ? align256(px * 4) : 0);
+    L.scratch_bytes = L.blob_tail_off + align256((long long)blob_k * sizeof(BlobAcc));
+    *out = L;
     return true;
-}
-
-__host__ inline long long plan_arena_bytes(const SmemPlan& p) {
-    return ((long long)p.gray_bytes + (long long)kNumMasks * p.mask_bytes + p.ws_bytes + 255) & ~255ll;
 }
 
 struct KArgs {
@@ -228,11 +287,7 @@ struct KArgs {
     long long* stats_out;           // compat modes: [n_total][4]
     int mode;
     int erode_r;                    // MODE_ERODE radius
-    uint8_t* scratch;               // per-CTA global scratch (general blur path, run-table overflow)
-    long long scratch_stride;
-    long long scratch_f32_off;      // offset of the float plane inside a CTA's scratch (adaptive threshold only)
-    long long scratch_rank_off;     // offset of the rank-count lists (dirty cells, ambiguous pixels)
-    int wmax, hmax;
+    uint8_t* scratch;               // per-CTA global scratch, layout.scratch_bytes apart
     long long* seg_stats;           // optional: [n_total][3] area, sum x, sum y of the final seg mask (CSV export), or null
     uint32_t* seg_bits;             // optional packed-bit masks (1 bit per pixel, rows of wpr words, PNG bit order), or null
     uint32_t* def_bits;
@@ -242,13 +297,12 @@ struct KArgs {
     int image_mul;                  //  a rank's shard of a multi-GPU job: global index = rank + k * world)
     vi_unit_record* peer_rec[kMaxPeers];   // record tables of all ranks (own included), peer-mapped: the record of global
     int n_peers;                    //  image g, unit u is stored at [g * n_units + u] of every one of them, or 0
-    uint8_t* arena;                 // GMEM kernel: per-CTA global arena holding what the shared-memory plan holds
-    long long arena_stride;         //  (gray crop, masks, workspace) for units larger than one SM's shared memory
+    uint8_t* arena;                 // GMEM kernel: per-CTA global arena (layout.arena_bytes apart) holding what shared
+                                    //  memory holds otherwise (gray crop, masks, workspace)
     long long* prof;                // diagnostics: [n_total][kProfSlots] per-phase cycle counts, or null
     vi_defect_blob* blobs;          // optional: [n_total][blob_k] kept defect components (vi_set_defect_blob_output), or null
     int blob_k;
-    long long scratch_blob_off;     // offset of the blob accumulators inside a CTA's scratch (tables beyond two masks)
-    SmemPlan plan;
+    UnitLayout layout;
     // Asynchronous crop gather through the tensor-memory accelerator (vi_pipeline.cuh: gather_issue_tma): the frames as
     // a 3-D uint8 tensor (x, y, image); one box = tma_bw x tma_bh pixels, a crop = tma_ncb x tma_nrb boxes that land as
     // tma_ncb dense tiles of row pitch tma_bw (tma_tile_bytes apart) in the staging area.
@@ -264,7 +318,7 @@ struct CtaScratch {
     // two buffers, used alternately: a collective writes its partials, passes ONE barrier and every warp reduces the
     // kWarps partials on its own; the next collective uses the other buffer, so no trailing barrier is needed (a warp
     // can only reach the call after next by passing the next call's barrier, i.e. after everybody's reads of this one).
-    // Kept small: every byte of static shared memory comes out of the histogram copies (vi_device.cuh: make_plan).
+    // Kept small: every byte of static shared memory comes out of the histogram copies (unit_layout).
     unsigned long long wl[2][2][kWarps];
     unsigned w32[2][kWarps];
     int flag;

@@ -62,20 +62,13 @@ struct RankWs {
     int plane_cap;       // words the plane holds (CHECKED builds)
 };
 
-constexpr int kExactCap = 4096;
 constexpr int kExactWarpMax = 192;       // more ambiguous pixels than this: one thread per pixel instead of one warp
-constexpr int kDirtyListCap = 4096, kExactListCap = 16384;     // rank_finish's lists in the labelling workspace hold at most these
-__host__ __device__ inline long long rank_plane_words(int wmax, int hmax) {
-    return (long long)rank_ngrp(wmax) * ((((hmax + kCell - 1) / kCell) + 15) & ~15);
-}
-__host__ __device__ inline long long rank_scratch_bytes(int wmax, int hmax) {
-    return rank_plane_words(wmax, hmax) * 4 + kExactCap * 4;
-}
 
 // The cell pass runs before the ROI exists (next to the Otsu scan), the per-pixel pass after it: the plane and the
 // list outlive the shared workspace, so they sit in the CTA's global scratch (L2-resident) and the counters in static
 // shared memory.
-__device__ inline RankWs rank_ws_carve(unsigned char* base, const Geom& g, unsigned char* lists, int wmax, int hmax, int* counters) {
+// `lists`: the plane of `plane_words` words, then kExactCap ambiguous pixels (vi_device.cuh: rank_scratch_bytes).
+__device__ inline RankWs rank_ws_carve(unsigned char* base, const Geom& g, unsigned char* lists, int plane_words, int* counters) {
     RankWs r;
     r.nlx = rank_nlx(g.w); r.nly = (g.h + kCell - 1) / kCell;
     r.ngrp = rank_ngrp(g.w); r.nrb = (r.nly + 15) >> 4;
@@ -85,7 +78,7 @@ __device__ inline RankWs rank_ws_carve(unsigned char* base, const Geom& g, unsig
     r.table = reinterpret_cast<unsigned*>(base);
     r.counters = counters;
     r.plane = reinterpret_cast<unsigned*>(lists);
-    r.plane_cap = (int)rank_plane_words(wmax, hmax);
+    r.plane_cap = plane_words;
     r.exact = r.plane + r.plane_cap;
     r.exact_cap = kExactCap;
     return r;

@@ -201,14 +201,14 @@ VI_PHASE int fill_holes(Cta& cta, unsigned* M, unsigned* T, const Geom& g, const
 // the general kernel is a constant here, so the non-default branches are not even in the code (a third of the
 // instructions, less pressure on the instruction cache and on registers).  The host picks it (vi_api.cu: launch_units).
 // GMEM: the instantiation for units beyond one SM's shared memory -- `smem` is then the CTA's arena in global memory
-// (same layout, make_plan_gmem) and `hist_smem` the shared-memory home of the histogram copies.
+// (same layout, vi_device.cuh: unit_layout) and `hist_smem` the shared-memory home of the histogram copies.
 template <bool PROF, bool SPEC, bool GMEM>
 __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned char* smem, unsigned char* hist_smem, UnitShared& sh, Cta& cta) {
     const int tid = threadIdx.x;
     const int img = uid / a.n_units, unit = uid - img * a.n_units;
     const int4 rc = a.rects[unit];
     const Geom g = make_geom(rc.z, rc.w);
-    const SmemPlan& plan = a.plan;
+    const UnitLayout& L = a.layout;
     const int npix = g.w * g.h;
     const int mode = SPEC ? (int)MODE_FULL : a.mode;
     const int cfg_blur_k = SPEC ? 3 : a.blur_k;
@@ -220,26 +220,19 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
     uint32_t* const cfg_def_bits = SPEC ? nullptr : a.def_bits;
 
     uint8_t* gray = smem;
-    unsigned char* Rg = smem + plan.gray_bytes;
-    unsigned* MA = reinterpret_cast<unsigned*>(Rg + 0 * plan.mask_bytes);
-    unsigned* MB = reinterpret_cast<unsigned*>(Rg + 1 * plan.mask_bytes);
-    unsigned* MC = reinterpret_cast<unsigned*>(Rg + 2 * plan.mask_bytes);
-    unsigned* MD = reinterpret_cast<unsigned*>(Rg + 3 * plan.mask_bytes);
-    unsigned* ME = reinterpret_cast<unsigned*>(Rg + 4 * plan.mask_bytes);
+    unsigned* MA = reinterpret_cast<unsigned*>(smem + L.gray_bytes + 0 * L.mask_bytes);
+    unsigned* MB = reinterpret_cast<unsigned*>(smem + L.gray_bytes + 1 * L.mask_bytes);
+    unsigned* MC = reinterpret_cast<unsigned*>(smem + L.gray_bytes + 2 * L.mask_bytes);
+    unsigned* MD = reinterpret_cast<unsigned*>(smem + L.gray_bytes + 3 * L.mask_bytes);
+    unsigned* ME = reinterpret_cast<unsigned*>(smem + L.gray_bytes + 4 * L.mask_bytes);
     unsigned* CAND = MC;                 // candidate mask of the median stage (ME when it could be zeroed early)
-    unsigned char* WS = Rg + kNumMasks * plan.mask_bytes;
+    unsigned char* WS = smem + L.ws_off;
 
-    // per-CTA global scratch: [u16 hsum][u8 blurred][run-table overflow]
-    unsigned char* gs = a.scratch + (long long)blockIdx.x * a.scratch_stride;
-    const long long maxpx = (long long)a.wmax * a.hmax;
-    const long long maxpx4 = (long long)((a.wmax + 3) & ~3) * a.hmax;      // blurred scratch rows are whole words
+    unsigned char* gs = a.scratch + (long long)blockIdx.x * L.scratch_bytes;
     unsigned short* g_hp = reinterpret_cast<unsigned short*>(gs);
-    uint8_t* g_blur = gs + ((maxpx * 2 + 15) & ~15ll);
-    unsigned char* g_ccl = g_blur + ((maxpx4 + 15) & ~15ll);
-    const int capg = a.hmax * (a.wmax / 2 + 1);
-    unsigned char* g_rank = gs + a.scratch_rank_off;
-    const CclWs ws_s = ccl_ws_carve(WS, plan.run_cap, a.hmax);
-    const CclWs ws_g = ccl_ws_carve(g_ccl, capg, a.hmax);
+    uint8_t* g_blur = gs + L.blur_off;
+    const CclWs ws_s = ccl_ws_carve(WS, L.run_cap, L.run_rf);
+    const CclWs ws_g = ccl_ws_carve(gs + L.runs_off, L.runs_cap, L.run_rf);
     CclWs ws;
 
     const long long moff = (long long)img * a.unit_px + a.unit_off[unit];
@@ -292,43 +285,41 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
         } else if (src_mode == 2) {
             blur_general(gray, g, cfg_blur_k, a.taps, g_hp, g_blur);
         }
-        unsigned* hist_base = reinterpret_cast<unsigned*>(GMEM ? hist_smem : Rg);
+        unsigned* hist_base = GMEM ? reinterpret_cast<unsigned*>(hist_smem) : MA;
         {
             uint4* h4 = reinterpret_cast<uint4*>(hist_base);                  // 128-bit stores: the copies are 16-byte aligned
-            for (int i = tid; i < plan.n_hist * (kHistWords / 4); i += kThreads) h4[i] = make_uint4(0u, 0u, 0u, 0u);
+            for (int i = tid; i < L.n_hist * (kHistWords / 4); i += kThreads) h4[i] = make_uint4(0u, 0u, 0u, 0u);
         }
         if (tid < 256) sh.hist[tid] = 0;
         if (tid == 0) sh.otsu_last = -1;              // "no bound yet" for the exact Otsu scan (vi_pipeline.cuh: otsu_scan)
         cta_sync();
         pt.acc(30);
-        if (SPEC || (src_mode == 1 && plan.n_hist >= kWarps / 2)) {
+        if (SPEC || (src_mode == 1 && hist_round_fits(L.n_hist))) {
             // default path: one histogram round on min(16, n_hist) warps
-            blur3_hist(gray, g, hist_base + warp_id() * kHistWords, min(plan.n_hist, kWarps));
+            blur3_hist(gray, g, hist_base + warp_id() * kHistWords, min(L.n_hist, kWarps));
             cta_sync();
             pt.acc(31);
-            hist_collect(hist_base, min(plan.n_hist, kWarps), sh.hist, false);
+            hist_collect(hist_base, min(L.n_hist, kWarps), sh.hist, false);
             cta_sync();
         } else {
-            for (int r0 = 0; r0 < kWarps; r0 += plan.n_hist) {
+            for (int r0 = 0; r0 < kWarps; r0 += L.n_hist) {
                 unsigned* hw = hist_base + (warp_id() - r0) * kHistWords;
-                if (src_mode == 0) blur_pass<0, true>(gray, g_blur, g, hw, sh.hist, r0, plan.n_hist, nullptr, 0);
-                else if (src_mode == 1) blur_pass<1, true>(gray, g_blur, g, hw, sh.hist, r0, plan.n_hist, nullptr, 0);
-                else blur_pass<2, true>(gray, g_blur, g, hw, sh.hist, r0, plan.n_hist, nullptr, 0);
+                if (src_mode == 0) blur_pass<0, true>(gray, g_blur, g, hw, sh.hist, r0, L.n_hist, nullptr, 0);
+                else if (src_mode == 1) blur_pass<1, true>(gray, g_blur, g, hw, sh.hist, r0, L.n_hist, nullptr, 0);
+                else blur_pass<2, true>(gray, g_blur, g, hw, sh.hist, r0, L.n_hist, nullptr, 0);
                 cta_sync();
-                hist_collect(hist_base, min(plan.n_hist, kWarps - r0), sh.hist, true);
+                hist_collect(hist_base, min(L.n_hist, kWarps - r0), sh.hist, true);
                 cta_sync();
             }
         }
         pt.tick();   // 1 blur + histogram
         // ---- P2: Otsu.  The exact scan is a serial recurrence in doubles: one warp runs it while the others walk the
         // columns of the median stage's cell pass, which needs no mask and only approximate levels (an approximate
-        // threshold splits the histogram into its classes).  The stage's workspace is the region of the masks after
-        // the first one: none of them is live before the threshold (the first holds a caller-supplied mask in
-        // MODE_DETECT).
-        double* ows = reinterpret_cast<double*>(WS + plan.ws_bytes - kOtsuWsBytes);
-        lattice = SPEC || ((mode == MODE_FULL || mode == MODE_DETECT) && cfg_defect_method == 0 &&
-                           rank_ws_bytes(g.w, g.h) + kOtsuWsBytes <= (long long)(kNumMasks - 1) * plan.mask_bytes + plan.ws_bytes);
-        RankWs rw = rank_ws_carve(Rg + plan.mask_bytes, g, g_rank, a.wmax, a.hmax, sh.rank_cnt);
+        // threshold splits the histogram into its classes).  The stage's lattice is not live before the threshold
+        // (the first mask, outside it, holds a caller-supplied mask in MODE_DETECT).
+        double* ows = reinterpret_cast<double*>(smem + L.otsu_off);
+        lattice = SPEC || ((mode == MODE_FULL || mode == MODE_DETECT) && cfg_defect_method == 0 && lattice_fits(g.w, g.h, L));
+        RankWs rw = rank_ws_carve(smem + L.lattice_off, g, gs + L.rank_off, L.rank_words, sh.rank_cnt);
         const bool vote = !SPEC && mode == MODE_DETECT && lattice;
         if (vote) { load_mask_bits(aux, g, MA); }       // the caller's mask decides which class the levels bracket
         // the exact Otsu scan starts now on its own warp when that warp owns no column of the cell pass
@@ -389,14 +380,14 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
         if (need_seg) {
             // ---- P3: inverse threshold ------------------------------------------
             if (adaptive)
-                adaptive_threshold(g_blur, g, a.adapt_bs, a.ataps, a.p.adapt_C, reinterpret_cast<float*>(gs + a.scratch_f32_off), MA);
+                adaptive_threshold(g_blur, g, a.adapt_bs, a.ataps, a.p.adapt_C, reinterpret_cast<float*>(gs + L.f32_off), MA);
             else if (src_mode == 0) blur_pass<0, false>(gray, g_blur, g, nullptr, nullptr, 0, kWarps, MA, otsu_t);
             else if (src_mode == 1) {
                 // (blurring again with the SWAR loop and comparing was measured: 25.7 k cycles against 17.5 k for this)
                 threshold_gray(gray, g, MB, otsu_t, sh.misc);
                 cta_sync();
                 pt.acc(29);
-                threshold_band(gray, g, MB, MA, MC, otsu_t, MD, 2 * (plan.mask_bytes / 4), sh.misc, pt);
+                threshold_band(gray, g, MB, MA, MC, otsu_t, reinterpret_cast<unsigned*>(smem + L.band_off), L.band_cap, sh.misc, pt);
             }
             else blur_pass<2, false>(gray, g_blur, g, nullptr, nullptr, 0, kWarps, MA, otsu_t);
             cta_sync();
@@ -556,17 +547,16 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
         cta_sync();
     }
     if (SPEC || lattice) {
-        RankWs rw = rank_ws_carve(Rg + plan.mask_bytes, g, g_rank, a.wmax, a.hmax, sh.rank_cnt);
+        RankWs rw = rank_ws_carve(smem + L.lattice_off, g, gs + L.rank_off, L.rank_words, sh.rank_cnt);
         // lists of the stage in the (free) labelling workspace: dirty cells of the ROI, ambiguous pixels
-        const int ccap = min(plan.ws_bytes >> 4, kDirtyListCap), ecap = min((plan.ws_bytes >> 2) - ccap, kExactListCap);
-        n_amb = rank_finish(gray, g, rw, sh.levels, thr, MD, CAND, reinterpret_cast<unsigned*>(WS), ccap,
-                            reinterpret_cast<unsigned*>(WS) + ccap, ecap, pt);
+        n_amb = rank_finish(gray, g, rw, sh.levels, thr, MD, CAND, reinterpret_cast<unsigned*>(WS), L.dirty_cap,
+                            reinterpret_cast<unsigned*>(WS) + L.dirty_cap, L.exact_cap, pt);
         if (SPEC) {
-            // the gray crop (and the first mask) are dead from here on: start the next unit's row copies into them
+            // the staging area is dead from here on: start the next unit's row copies into it
             const int nuid = uid + (int)gridDim.x;
             if (nuid < a.n_images * a.n_units)
-                cta.gpending = (a.tma_ok ? gather_issue_tma(a, nuid, smem, plan.gray_bytes + plan.mask_bytes, &sh.gather_mbar)
-                                         : gather_issue(a, nuid, smem, plan.gray_bytes + plan.mask_bytes, &sh.gather_mbar)) ? 1 : 0;
+                cta.gpending = (a.tma_ok ? gather_issue_tma(a, nuid, smem, L.stage_bytes, &sh.gather_mbar)
+                                         : gather_issue(a, nuid, smem, L.stage_bytes, &sh.gather_mbar)) ? 1 : 0;
         }
     } else {
         // units wider than the column-per-thread pass: exact rank count for every ROI pixel
@@ -629,13 +619,11 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
     ccl_paint(ME, nullptr, g, ws, keep);
     cta_sync();
     if (a.blobs && n_kept > 0) {
-        // the kept components as a table (vi_set_defect_blob_output): a run-time pointer, in every instantiation.  Its
-        // accumulators take MC and MD, dead from here on (MB was read by the area pass above, MA may be receiving the
-        // next unit's crop; in GMEM they are the arena's), or the CTA's global scratch when they do not fit there.
+        // the kept components as a table (vi_set_defect_blob_output): a run-time pointer, in every instantiation
         const int kc = min(n_kept, a.blob_k);
-        const int cap_m = 2 * plan.mask_bytes / (int)sizeof(BlobAcc);
-        BlobAcc* tab = kc <= cap_m ? reinterpret_cast<BlobAcc*>(MC) : reinterpret_cast<BlobAcc*>(gs + a.scratch_blob_off);
-        ccl_blob_table(cta, ws, R, keep, kc, kc <= cap_m ? cap_m : a.blob_k, tab, a.blobs + (long long)uid * a.blob_k);
+        const bool in_masks = kc <= L.blob_cap;
+        BlobAcc* tab = reinterpret_cast<BlobAcc*>(in_masks ? smem + L.blob_off : gs + L.blob_tail_off);
+        ccl_blob_table(cta, ws, R, keep, kc, in_masks ? L.blob_cap : a.blob_k, tab, a.blobs + (long long)uid * a.blob_k);
     }
     pt.tick();   // 14 component area filter (+ blob table)
     // ---- P14: verdict ---------------------------------------------------------
@@ -667,9 +655,9 @@ __global__ void __launch_bounds__(kThreads, 1) vi_unit_kernel(const __grid_const
         if (threadIdx.x == 0) mbar_init(&sh.gather_mbar, 1u);
         cta_sync();
     }
-    unsigned char* base = GMEM ? a.arena + (long long)blockIdx.x * a.arena_stride : smem;
+    unsigned char* base = GMEM ? a.arena + (long long)blockIdx.x * a.layout.arena_bytes : smem;
     if (SPEC && a.tma_ok && (int)blockIdx.x < n_total)           // the first unit's crop arrives the same way as the later ones
-        cta.gpending = gather_issue_tma(a, blockIdx.x, smem, a.plan.gray_bytes + a.plan.mask_bytes, &sh.gather_mbar) ? 1 : 0;
+        cta.gpending = gather_issue_tma(a, blockIdx.x, smem, a.layout.stage_bytes, &sh.gather_mbar) ? 1 : 0;
     for (int uid = blockIdx.x; uid < n_total; uid += gridDim.x) {
         process_unit<PROF, SPEC, GMEM>(a, uid, base, smem, sh, cta);
         cta_sync();
