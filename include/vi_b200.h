@@ -14,15 +14,15 @@
  * There is no CPU fallback: every compute entry point runs CUDA kernels on the
  * context's device and fails with VI_ERR_CUDA if it cannot.
  *
- * Threading: one vi_ctx per host thread and device.  vi_inspect_batch is
- * asynchronous with respect to `stream`; all *_host / compat entry points
- * block until their results are in the caller's host buffers.
+ * Threading: one vi_ctx per host thread and device.  vi_inspect_batch and
+ * vi_segment_batch are asynchronous with respect to `stream`; all *_host /
+ * compat entry points block until their results are in the caller's host buffers.
  *
  * Ordering: a context's tables (grid, exclusions, reference centroids) and its
  * per-SM scratch are shared by all of its calls.  The library orders them
  * itself: every entry point waits (on the device for a stream launch, on the host
  * for a table update or a blocking call) for the last asynchronous
- * vi_inspect_batch of the same context before touching them, whatever stream that
+ * vi_inspect_batch / vi_segment_batch of the same context before touching them, whatever stream that
  * batch ran on.  Output buffers of an asynchronous batch stay the caller's to
  * synchronise.  Every entry point leaves the caller's current CUDA device as it
  * found it.
@@ -46,6 +46,7 @@ extern "C" {
 #define VI_STATUS_OK 0        /* detector returned None or area < min_area (indexing_ui.py:1687, :1699) */
 #define VI_STATUS_NG 1        /* defect area >= min_area (indexing_ui.py:1618, :1699)                   */
 #define VI_STATUS_ROI_EMPTY 2 /* ROI empty after erosion -> detector returns None (:1514-1516)          */
+#define VI_STATUS_SEGMENTED 3 /* segmented only (vi_segment_batch): no detector ran, no verdict          */
 
 typedef struct vi_ctx vi_ctx;
 
@@ -176,6 +177,23 @@ int vi_inspect_batch_host_blobs(vi_ctx* ctx, const uint8_t* h_frames, int n_imag
                                 int64_t row_pitch, int64_t image_stride, const vi_params* params,
                                 int mask_format, void* h_seg_masks, void* h_defect_masks,
                                 vi_unit_record* h_records, vi_defect_blob* h_blobs, int max_per_unit);
+
+/* Segmentation only: run_segmentation_all (indexing_ui.py:2203-2368) for every unit of every image, without the
+ * defect detector -- what an image switch, an exclusion edit, the reference image's centroids
+ * (exclusion_alignment.ref_centroids, :2214-2233) and the mask / CSV export (:2703-2730) need.  Arguments, argument
+ * errors, frames, grid, exclusions, reference centroids, seg-mask packing and the peer record tables are those of
+ * vi_inspect_batch; so are the vi_set_seg_stats_output and vi_set_packed_mask_output seg outputs.  Records: otsu_t,
+ * seg_area, dx, dy, cx, cy and n_runs as vi_inspect_batch gives them; roi_area, defect_area, n_kept and n_ambiguous
+ * are 0; status is VI_STATUS_SEGMENTED.  The defect bits, the blob table and labels are never written.
+ * Asynchronous on `stream`. */
+int vi_segment_batch(vi_ctx* ctx, const uint8_t* d_frames, int n_images, int W, int H, int64_t row_pitch,
+                     int64_t image_stride, const vi_params* params, uint8_t* d_seg_masks, vi_unit_record* d_records,
+                     void* stream);
+/* vi_segment_batch from and to HOST buffers, as vi_inspect_batch_host_fmt does it (chunks on internal streams, the
+ * covered rows uploaded, VI_MASKS_* formats; h_seg_masks may be NULL).  Blocks until done. */
+int vi_segment_batch_host(vi_ctx* ctx, const uint8_t* h_frames, int n_images, int W, int H, int64_t row_pitch,
+                          int64_t image_stride, const vi_params* params, int mask_format, void* h_seg_masks,
+                          vi_unit_record* h_records);
 
 /* Packed-bit masks (VI_MASKS_PACKED layout) as an optional extra output of subsequent vi_inspect_batch calls:
  * device pointers, vi_packed_mask_bytes per image; NULL switches one off. */

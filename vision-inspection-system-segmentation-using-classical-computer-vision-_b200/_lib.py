@@ -11,7 +11,7 @@ from . import _build
 
 VI_OK = 0
 VI_ERR_ARG, VI_ERR_CUDA, VI_ERR_UNSUPPORTED, VI_ERR_TOO_LARGE = -1, -2, -3, -4
-STATUS_OK, STATUS_NG, STATUS_ROI_EMPTY = 0, 1, 2
+STATUS_OK, STATUS_NG, STATUS_ROI_EMPTY, STATUS_SEGMENTED = 0, 1, 2, 3
 MASKS_BYTES, MASKS_PACKED, MASKS_NONE = 0, 1, 2
 
 
@@ -42,7 +42,7 @@ MAX_BLOBS_PER_UNIT = 1024
 EXPORTS = [
     "vi_last_error", "vi_version", "vi_params_default", "vi_ctx_create", "vi_ctx_destroy", "vi_set_grid",
     "vi_set_exclusions", "vi_set_ref_centroids", "vi_unit_pixels", "vi_unit_offsets", "vi_inspect_batch",
-    "vi_inspect_batch_host", "vi_inspect_batch_host_fmt", "vi_inspect_batch_host_blobs", "vi_set_defect_blob_output", "vi_set_packed_mask_output", "vi_packed_mask_bytes",
+    "vi_inspect_batch_host", "vi_inspect_batch_host_fmt", "vi_inspect_batch_host_blobs", "vi_segment_batch", "vi_segment_batch_host", "vi_set_defect_blob_output", "vi_set_packed_mask_output", "vi_packed_mask_bytes",
     "vi_packed_mask_offsets", "vi_host_upload_bytes", "vi_peer_table_create", "vi_peer_table_open", "vi_peer_table_close",
     "vi_peer_table_destroy", "vi_peer_table_read", "vi_set_record_peers", "vi_segment_cell", "vi_fill_internal_holes", "vi_mask_stats", "vi_erode_square",
     "vi_label_components", "vi_detect_defects", "vi_ingest_argb32", "vi_ingest_gray16", "vi_set_seg_stats_output", "vi_debug_set_profile", "vi_debug_check_word", "vi_debug_fastdiv_check", "vi_debug_otsu",
@@ -91,6 +91,8 @@ def load():
     lib.vi_inspect_batch_host_fmt.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, i64, i64, P(ViParams), C.c_int, vp, vp, vp]
     lib.vi_inspect_batch_host_blobs.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, i64, i64, P(ViParams), C.c_int, vp, vp, vp,
                                                 vp, C.c_int]
+    lib.vi_segment_batch.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, i64, i64, P(ViParams), vp, vp, vp]
+    lib.vi_segment_batch_host.argtypes = [vp, vp, C.c_int, C.c_int, C.c_int, i64, i64, P(ViParams), C.c_int, vp, vp]
     lib.vi_set_packed_mask_output.argtypes = [vp, vp, vp]
     lib.vi_set_defect_blob_output.argtypes = [vp, vp, C.c_int]
     lib.vi_packed_mask_bytes.argtypes = [vp]

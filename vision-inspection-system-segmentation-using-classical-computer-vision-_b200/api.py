@@ -151,6 +151,39 @@ class Inspector:
             labels.data_ptr() if labels is not None else None, records.data_ptr(), C.c_void_p(st.cuda_stream)))
         return records, seg_masks, defect_masks
 
+    def segment_batch(self, frames, params=None, seg_masks=None, records=None, stream=None, seg_stats=None, seg_bits=None):
+        """run_segmentation_all for every unit of every frame, without the defect detector.  frames as for
+        `inspect_batch`; returns (records, seg_masks) as CUDA tensors, asynchronous on `stream`.  Records carry otsu_t,
+        seg_area, dx, dy, cx, cy (the pre-exclusion centroid: `grid.ref_centroids_from_records`) and status
+        STATUS_SEGMENTED; the detector's fields are 0.  seg_stats / seg_bits: optional outputs as in `inspect_batch`."""
+        import torch
+        if not frames.is_cuda or frames.dtype != torch.uint8 or frames.dim() != 3:
+            raise TypeError("frames must be a CUDA uint8 tensor [n, H, W]")
+        if frames.stride(2) != 1:
+            raise ValueError("frames must be contiguous along x")
+        n, H, W = frames.shape
+        dev = frames.device
+        if dev.index != self.device:
+            raise ValueError(f"frames are on {dev}, this Inspector drives cuda:{self.device}")
+        total = n * self.unit_pixels
+        self._check_out(seg_masks, "seg_masks", dev, torch.uint8, total)
+        self._check_out(records, "records", dev, torch.uint8, n * self.n_units * 64)
+        self._check_out(seg_stats, "seg_stats", dev, torch.int64, n * self.n_units * 3)
+        self._check_out(seg_bits, "seg_bits", dev, torch.uint8, n * self.packed_bytes)
+        if seg_masks is None:
+            seg_masks = torch.empty(total, dtype=torch.uint8, device=dev)
+        if records is None:
+            records = torch.empty((n * self.n_units, 64), dtype=torch.uint8, device=dev)
+        st = stream if stream is not None else torch.cuda.current_stream(dev)
+        p = params if params is not None else default_params()
+        check(self._lib.vi_set_seg_stats_output(self._ctx, seg_stats.data_ptr() if seg_stats is not None else None))
+        check(self._lib.vi_set_packed_mask_output(self._ctx, seg_bits.data_ptr() if seg_bits is not None else None, None))
+        check(self._lib.vi_segment_batch(
+            self._ctx, frames.data_ptr(), int(n), int(W), int(H), int(frames.stride(1)),
+            int(frames.stride(0)) if n > 1 else int(frames.stride(1)) * int(H),
+            C.byref(p), seg_masks.data_ptr(), records.data_ptr(), C.c_void_p(st.cuda_stream)))
+        return records, seg_masks
+
     # ---- frame ingest (device) -------------------------------------------------------
     def ingest_argb32(self, frames_bgra, out=None, stream=None):
         """QImage ARGB32 frames (CUDA uint8 [n, H, W, 4], bytes B,G,R,A) -> mono CUDA uint8 [n, H, W], the reference's
@@ -231,6 +264,23 @@ class Inspector:
             seg.ctypes.data if seg is not None else None, dfm.ctypes.data if dfm is not None else None,
             rec.ctypes.data))
         return rec, seg, dfm
+
+    def segment_batch_host(self, frames: np.ndarray, params=None, mask_format="bytes"):
+        """`segment_batch` from and to host arrays (frames uint8 [n, H, W]), pipelined as `inspect_batch_host` is.
+        mask_format: "bytes", "packed" or "none".  Returns (records structured array, seg_masks u8 | None)."""
+        frames = _u8c(frames, "frames")
+        if frames.ndim != 3:
+            raise ValueError("frames must be [n, H, W]")
+        n, H, W = frames.shape
+        fmt = {"bytes": _lib.MASKS_BYTES, "packed": _lib.MASKS_PACKED, "none": _lib.MASKS_NONE}[mask_format]
+        per_image = {_lib.MASKS_BYTES: self.unit_pixels, _lib.MASKS_PACKED: self.packed_bytes, _lib.MASKS_NONE: 0}[fmt]
+        rec = np.empty(n * self.n_units, RECORD_DTYPE)
+        seg = np.empty(n * per_image, np.uint8) if fmt != _lib.MASKS_NONE else None
+        p = params if params is not None else default_params()
+        check(self._lib.vi_segment_batch_host(
+            self._ctx, frames.ctypes.data, int(n), int(W), int(H), int(W), int(H) * int(W), C.byref(p), fmt,
+            seg.ctypes.data if seg is not None else None, rec.ctypes.data))
+        return rec, seg
 
     def kept_blobs(self, records, blobs, image, unit):
         """The valid kept-component entries of one (image, unit): records (RECORD_DTYPE, [n*units] or [n, units]) and a

@@ -776,7 +776,9 @@ static int launch_units(vi_ctx* c, KArgs& a, const GridState& gs, cudaStream_t s
         CU(cudaFuncSetAttribute(vi_unit_kernel<false, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
 #ifndef VI_CHECKED
         CU(cudaFuncSetAttribute(vi_unit_kernel<true, true, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
+        CU(cudaFuncSetAttribute(vi_seg_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
 #endif
+        CU(cudaFuncSetAttribute(vi_seg_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
         CU(cudaFuncSetAttribute(vi_unit_kernel<false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, lim));
         c->smem_set = lim;
     }
@@ -788,17 +790,21 @@ static int launch_units(vi_ctx* c, KArgs& a, const GridState& gs, cudaStream_t s
         CU(cudaGetLastError());
         return VI_OK;
     }
-    // The default configuration has its own instantiation (vi_unit.cuh: SPEC).
+    // The default configuration has its own instantiations (vi_unit.cuh: SPEC), one per batch mode.
+    const bool aligned = (a.row_pitch & 15) == 0 && (reinterpret_cast<uintptr_t>(a.frames) & 15) == 0 && (a.image_stride & 15) == 0;
     bool spec = a.mode == MODE_FULL && a.blur_k == 3 && a.se_k == 3 && a.p.seg_method == 0 && a.p.defect_method == 0 &&
-                !a.labels_out && !a.seg_stats && !a.seg_bits && !a.def_bits && !a.aux_mask && !a.stats_out &&
-                (a.row_pitch & 15) == 0 && (reinterpret_cast<uintptr_t>(a.frames) & 15) == 0 && (a.image_stride & 15) == 0 &&
+                !a.labels_out && !a.seg_stats && !a.seg_bits && !a.def_bits && !a.aux_mask && !a.stats_out && aligned &&
                 lattice_fits(gs.ext.wmax, gs.ext.hmax, L) && hist_round_fits(L.n_hist);
-    if (spec) make_frame_tensor(a, gs);
+    const bool seg = a.mode == MODE_SEG_ONLY && a.blur_k == 3 && a.se_k == 3 && a.p.seg_method == 0 && !a.labels_out &&
+                     !a.def_bits && !a.aux_mask && !a.stats_out && aligned && hist_round_fits(L.n_hist);
+    if (spec || seg) make_frame_tensor(a, gs);
 #ifndef VI_CHECKED
     if (a.prof && spec) vi_unit_kernel<true, true, false><<<nblocks, kThreads, L.total, stream>>>(a);   // diagnostics build: phase timers
+    else if (a.prof && seg) vi_seg_kernel<true><<<nblocks, kThreads, L.total, stream>>>(a);
     else
 #endif
     if (spec) vi_unit_kernel<false, true, false><<<nblocks, kThreads, L.total, stream>>>(a);
+    else if (seg) vi_seg_kernel<false><<<nblocks, kThreads, L.total, stream>>>(a);
     else { a.prof = nullptr; vi_unit_kernel<false, false, false><<<nblocks, kThreads, L.total, stream>>>(a); }
     CU(cudaGetLastError());
     return VI_OK;
@@ -839,12 +845,14 @@ static void batch_args(vi_ctx* c, KArgs& a, const uint8_t* frames, int n_images,
     a.prof = c->prof;
 }
 
-extern "C" int vi_inspect_batch(vi_ctx* c, const uint8_t* d_frames, int n_images, int W, int H, int64_t row_pitch,
-                                int64_t image_stride, const vi_params* params, uint8_t* d_seg, uint8_t* d_def,
-                                int32_t* d_labels, vi_unit_record* d_rec, void* stream) {
+// The device-buffer batch call in `mode`: MODE_FULL (vi_inspect_batch) or MODE_SEG_ONLY (vi_segment_batch, which
+// takes no defect, label or blob outputs).
+static int device_batch(vi_ctx* c, int mode, const char* name, const uint8_t* d_frames, int n_images, int W, int H,
+                        int64_t row_pitch, int64_t image_stride, const vi_params* params, uint8_t* d_seg, uint8_t* d_def,
+                        int32_t* d_labels, vi_unit_record* d_rec, void* stream) {
     if (!c) return fail(VI_ERR_ARG, "ctx is null");
-    if (c->grid.rects.empty()) return fail(VI_ERR_ARG, "vi_inspect_batch: no grid set");
-    if (!d_frames || !d_rec) return fail(VI_ERR_ARG, "vi_inspect_batch: frames / records pointer is null");
+    if (c->grid.rects.empty()) return fail(VI_ERR_ARG, "%s: no grid set", name);
+    if (!d_frames || !d_rec) return fail(VI_ERR_ARG, "%s: frames / records pointer is null", name);
     if (n_images == 1 && image_stride < row_pitch * (int64_t)H) image_stride = row_pitch * (int64_t)H;
     VI_DEVICE(c);
     int rc;
@@ -853,10 +861,14 @@ extern "C" int vi_inspect_batch(vi_ctx* c, const uint8_t* d_frames, int n_images
     base_args(c, a, c->grid);
     if ((rc = fill_params(a, params))) return rc;
     batch_args(c, a, d_frames, n_images, W, H, row_pitch, image_stride);
-    a.seg_out = d_seg; a.def_out = d_def; a.labels_out = d_labels; a.rec = d_rec;
+    a.mode = mode;
+    a.seg_out = d_seg; a.rec = d_rec;
     a.seg_stats = c->seg_stats;
-    a.seg_bits = c->seg_bits; a.def_bits = c->def_bits;
-    a.blobs = c->blobs; a.blob_k = c->blob_k;
+    a.seg_bits = c->seg_bits;
+    if (mode == MODE_FULL) {
+        a.def_out = d_def; a.labels_out = d_labels; a.def_bits = c->def_bits;
+        a.blobs = c->blobs; a.blob_k = c->blob_k;
+    }
     a.n_peers = c->n_peers; a.image_mul = c->image_mul; a.image_base = c->image_add;
     for (int i = 0; i < c->n_peers; ++i) a.peer_rec[i] = c->peer_rec[i];
     if ((rc = wait_busy_stream(c, (cudaStream_t)stream))) return rc;     // an earlier batch on another stream shares the scratch
@@ -864,15 +876,31 @@ extern "C" int vi_inspect_batch(vi_ctx* c, const uint8_t* d_frames, int n_images
     return mark_busy(c, (cudaStream_t)stream);
 }
 
+extern "C" int vi_inspect_batch(vi_ctx* c, const uint8_t* d_frames, int n_images, int W, int H, int64_t row_pitch,
+                                int64_t image_stride, const vi_params* params, uint8_t* d_seg, uint8_t* d_def,
+                                int32_t* d_labels, vi_unit_record* d_rec, void* stream) {
+    return device_batch(c, MODE_FULL, "vi_inspect_batch", d_frames, n_images, W, H, row_pitch, image_stride, params, d_seg,
+                        d_def, d_labels, d_rec, stream);
+}
+
+extern "C" int vi_segment_batch(vi_ctx* c, const uint8_t* d_frames, int n_images, int W, int H, int64_t row_pitch,
+                                int64_t image_stride, const vi_params* params, uint8_t* d_seg, vi_unit_record* d_rec,
+                                void* stream) {
+    return device_batch(c, MODE_SEG_ONLY, "vi_segment_batch", d_frames, n_images, W, H, row_pitch, image_stride, params,
+                        d_seg, nullptr, nullptr, d_rec, stream);
+}
+
 // Host-buffer batch call.  mask_format: VI_MASKS_BYTES (0/255 bytes, what the reference's pixmaps hold),
 // VI_MASKS_PACKED (1 bit per pixel, rows of 32-bit words, PNG bit order) or VI_MASKS_NONE (records only: all that
-// run_inspection needs, indexing_ui.py:1686-1706).
-static int host_batch(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, int H, int64_t row_pitch, int64_t image_stride,
-                      const vi_params* params, int mask_format, void* h_seg, void* h_def, vi_unit_record* h_rec,
-                      vi_defect_blob* h_blobs = nullptr, int blob_k = 0) {
+// run_inspection needs, indexing_ui.py:1686-1706).  mode: MODE_FULL, or MODE_SEG_ONLY (vi_segment_batch_host: no
+// defect masks, no blob table).
+static int host_batch(vi_ctx* c, int mode, const uint8_t* h_frames, int n_images, int W, int H, int64_t row_pitch,
+                      int64_t image_stride, const vi_params* params, int mask_format, void* h_seg, void* h_def,
+                      vi_unit_record* h_rec, vi_defect_blob* h_blobs = nullptr, int blob_k = 0) {
+    const char* name = mode == MODE_SEG_ONLY ? "vi_segment_batch_host" : "vi_inspect_batch_host";
     if (!c) return fail(VI_ERR_ARG, "ctx is null");
-    if (c->grid.rects.empty()) return fail(VI_ERR_ARG, "vi_inspect_batch_host: no grid set");
-    if (!h_frames || !h_rec) return fail(VI_ERR_ARG, "vi_inspect_batch_host: frames / records pointer is null");
+    if (c->grid.rects.empty()) return fail(VI_ERR_ARG, "%s: no grid set", name);
+    if (!h_frames || !h_rec) return fail(VI_ERR_ARG, "%s: frames / records pointer is null", name);
     if (mask_format < VI_MASKS_BYTES || mask_format > VI_MASKS_NONE) return fail(VI_ERR_ARG, "mask_format %d", mask_format);
     if (h_blobs && (blob_k < 1 || blob_k > VI_MAX_BLOBS_PER_UNIT))
         return fail(VI_ERR_ARG, "vi_inspect_batch_host_blobs: %d blobs per unit (1..%d)", blob_k, VI_MAX_BLOBS_PER_UNIT);
@@ -888,6 +916,7 @@ static int host_batch(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, i
     const long long upx = c->grid.unit_px;
     const long long ubytes = mask_format == VI_MASKS_BYTES ? upx : mask_format == VI_MASKS_PACKED ? c->grid.unit_words * 4 : 0;
     if (mask_format == VI_MASKS_NONE) { h_seg = nullptr; h_def = nullptr; }
+    if (mode == MODE_SEG_ONLY) { h_def = nullptr; h_blobs = nullptr; }
     // Chunks of about two units per SM, kHostSlots of them in flight: the call is bound by the host link (frames up,
     // masks down), so all that matters is that the copy engines never idle.  VI_HOST_CHUNK overrides (images per chunk).
     int chunk = std::max(1, (2 * c->sm_count + n_units - 1) / n_units);
@@ -917,6 +946,7 @@ static int host_batch(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, i
             }
             KArgs a = a0;
             batch_args(c, a, (const uint8_t*)c->hb_frames[slot].p, n, W, H, row_pitch, image_stride);
+            a.mode = mode;
             a.image_base = i0;
             if (mask_format == VI_MASKS_BYTES) {
                 a.seg_out = h_seg ? (uint8_t*)c->hb_seg[slot].p : nullptr; a.def_out = h_def ? (uint8_t*)c->hb_def[slot].p : nullptr;
@@ -950,20 +980,27 @@ static int host_batch(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, i
 extern "C" int vi_inspect_batch_host(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, int H, int64_t row_pitch,
                                      int64_t image_stride, const vi_params* params, uint8_t* h_seg, uint8_t* h_def,
                                      vi_unit_record* h_rec) {
-    return host_batch(c, h_frames, n_images, W, H, row_pitch, image_stride, params, VI_MASKS_BYTES, h_seg, h_def, h_rec);
+    return host_batch(c, MODE_FULL, h_frames, n_images, W, H, row_pitch, image_stride, params, VI_MASKS_BYTES, h_seg, h_def, h_rec);
 }
 
 extern "C" int vi_inspect_batch_host_fmt(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, int H, int64_t row_pitch,
                                          int64_t image_stride, const vi_params* params, int mask_format, void* h_seg,
                                          void* h_def, vi_unit_record* h_rec) {
-    return host_batch(c, h_frames, n_images, W, H, row_pitch, image_stride, params, mask_format, h_seg, h_def, h_rec);
+    return host_batch(c, MODE_FULL, h_frames, n_images, W, H, row_pitch, image_stride, params, mask_format, h_seg, h_def, h_rec);
 }
 
 extern "C" int vi_inspect_batch_host_blobs(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, int H, int64_t row_pitch,
                                            int64_t image_stride, const vi_params* params, int mask_format, void* h_seg,
                                            void* h_def, vi_unit_record* h_rec, vi_defect_blob* h_blobs, int max_per_unit) {
-    return host_batch(c, h_frames, n_images, W, H, row_pitch, image_stride, params, mask_format, h_seg, h_def, h_rec,
+    return host_batch(c, MODE_FULL, h_frames, n_images, W, H, row_pitch, image_stride, params, mask_format, h_seg, h_def, h_rec,
                       h_blobs, max_per_unit);
+}
+
+extern "C" int vi_segment_batch_host(vi_ctx* c, const uint8_t* h_frames, int n_images, int W, int H, int64_t row_pitch,
+                                     int64_t image_stride, const vi_params* params, int mask_format, void* h_seg,
+                                     vi_unit_record* h_rec) {
+    return host_batch(c, MODE_SEG_ONLY, h_frames, n_images, W, H, row_pitch, image_stride, params, mask_format, h_seg, nullptr,
+                      h_rec);
 }
 
 // ---------------------------------------------------------------------------

@@ -171,6 +171,8 @@ struct UnitExtent {
 //             not fit, the scratch blob tail
 //   stage     the next unit's crop gather, from rank_finish (P11) on (shared-memory kernel);  gray, MA (the ROI pass
 //             is done with both)
+//   stage, segmentation kernel: from the first close pass on (P4: the passes alternate MB / MC after reading MA,
+//             and the hole fill, centroid, exclusions and stores work on MC);  gray, MA
 // Per-CTA scratch in global memory (scratch_bytes apart, L2-resident), no aliases:
 //   [ u16 hsum | u8 blurred (rows of whole words) | run-table overflow | rank plane + exact list | f32 plane | blobs ]
 struct UnitLayout {

@@ -200,9 +200,12 @@ VI_PHASE int fill_holes(Cta& cta, unsigned* M, unsigned* T, const Geom& g, const
 // method, lattice rank stage, 16-byte aligned frames, no optional outputs): everything that is a run-time choice in
 // the general kernel is a constant here, so the non-default branches are not even in the code (a third of the
 // instructions, less pressure on the instruction cache and on registers).  The host picks it (vi_api.cu: launch_units).
+// SPEC && SEG: the same configuration in the segmentation-only mode (vi_segment_batch): no detector, and the seg_stats
+// and packed seg-bit outputs stay run-time pointers (the mask export needs them).  The mask is carried in MB / MC from
+// the first close pass on, so that the next unit's crop can be gathered into gray and MA from there.
 // GMEM: the instantiation for units beyond one SM's shared memory -- `smem` is then the CTA's arena in global memory
 // (same layout, vi_device.cuh: unit_layout) and `hist_smem` the shared-memory home of the histogram copies.
-template <bool PROF, bool SPEC, bool GMEM>
+template <bool PROF, bool SPEC, bool GMEM, bool SEG>
 __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned char* smem, unsigned char* hist_smem, UnitShared& sh, Cta& cta) {
     const int tid = threadIdx.x;
     const int img = uid / a.n_units, unit = uid - img * a.n_units;
@@ -210,13 +213,13 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
     const Geom g = make_geom(rc.z, rc.w);
     const UnitLayout& L = a.layout;
     const int npix = g.w * g.h;
-    const int mode = SPEC ? (int)MODE_FULL : a.mode;
+    const int mode = SPEC ? (SEG ? (int)MODE_SEG_ONLY : (int)MODE_FULL) : a.mode;
     const int cfg_blur_k = SPEC ? 3 : a.blur_k;
     const int cfg_se_k = SPEC ? 3 : a.se_k;
     const int cfg_seg_method = SPEC ? 0 : a.p.seg_method;
     const int cfg_defect_method = SPEC ? 0 : a.p.defect_method;
-    long long* const cfg_seg_stats = SPEC ? nullptr : a.seg_stats;
-    uint32_t* const cfg_seg_bits = SPEC ? nullptr : a.seg_bits;
+    long long* const cfg_seg_stats = SPEC && !SEG ? nullptr : a.seg_stats;
+    uint32_t* const cfg_seg_bits = SPEC && !SEG ? nullptr : a.seg_bits;
     uint32_t* const cfg_def_bits = SPEC ? nullptr : a.def_bits;
 
     uint8_t* gray = smem;
@@ -318,7 +321,7 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
         // threshold splits the histogram into its classes).  The stage's lattice is not live before the threshold
         // (the first mask, outside it, holds a caller-supplied mask in MODE_DETECT).
         double* ows = reinterpret_cast<double*>(smem + L.otsu_off);
-        lattice = SPEC || ((mode == MODE_FULL || mode == MODE_DETECT) && cfg_defect_method == 0 && lattice_fits(g.w, g.h, L));
+        lattice = (SPEC && !SEG) || ((mode == MODE_FULL || mode == MODE_DETECT) && cfg_defect_method == 0 && lattice_fits(g.w, g.h, L));
         RankWs rw = rank_ws_carve(smem + L.lattice_off, g, gs + L.rank_off, L.rank_words, sh.rank_cnt);
         const bool vote = !SPEC && mode == MODE_DETECT && lattice;
         if (vote) { load_mask_bits(aux, g, MA); }       // the caller's mask decides which class the levels bracket
@@ -399,7 +402,19 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
                 CAND = ME;
             }
             // ---- P4: close, open --------------------------------------------------
-            if (cfg_se_k == 3) {
+            unsigned* S = MA;                                // the seg mask from here on
+            if (SPEC && SEG) {
+                cross3_pass<false>(MA, MB, g); cta_sync();
+                // gray and MA are dead: the next unit's crop goes into the staging area over them meanwhile
+                const int nuid = uid + (int)gridDim.x;
+                if (nuid < a.n_images * a.n_units)
+                    cta.gpending = (a.tma_ok ? gather_issue_tma(a, nuid, smem, L.stage_bytes, &sh.gather_mbar)
+                                             : gather_issue(a, nuid, smem, L.stage_bytes, &sh.gather_mbar)) ? 1 : 0;
+                cross3_pass<true>(MB, MC, g); cta_sync();
+                cross3_pass<true>(MC, MB, g); cta_sync();
+                cross3_pass<false>(MB, MC, g); cta_sync();
+                S = MC;
+            } else if (cfg_se_k == 3) {
                 cross3_pass<false>(MA, MB, g); cta_sync();
                 cross3_pass<true>(MB, MA, g); cta_sync();
                 cross3_pass<true>(MA, MB, g); cta_sync();
@@ -413,20 +428,20 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
             pt.tick();   // 5 close/open
             // ---- P5: hole fill ----------------------------------------------------
             unsigned* rowinfo = reinterpret_cast<unsigned*>(ws_s.row_first());
-            RowScan rs = mask_row_scan(cta, MA, g, rowinfo);
+            RowScan rs = mask_row_scan(cta, S, g, rowinfo);
             if (rs.any_multi) {                              // a row with several runs: the background may have holes
                 int how = 0;
-                n_runs_max = max(n_runs_max, fill_holes(cta, MA, MB, g, ws_s, ws_g, ws, &pt, &how));
-                if (mode == MODE_FULL) rs = how == 2 ? mask_row_rescan_filled(cta, MA, g, rowinfo) : mask_row_scan(cta, MA, g, rowinfo);
+                n_runs_max = max(n_runs_max, fill_holes(cta, S, MB, g, ws_s, ws_g, ws, &pt, &how));
+                rs = how == 2 ? mask_row_rescan_filled(cta, S, g, rowinfo) : mask_row_scan(cta, S, g, rowinfo);
             }
             pt.tick();   // 6 hole fill
-            if (mode == MODE_FULL) {
+            {
                 // ---- P6: largest 8-component centroid, shift ---------------------
                 unsigned area; unsigned long long sx, sy;
                 int broot = 1;
                 if (rs.solid) { area = rs.area; sx = rs.sx; sy = rs.sy; }
                 else {
-                    const int R = ccl_build(cta, MA, g, true, false, ws_s, ws_g, ws, &pt);
+                    const int R = ccl_build(cta, S, g, true, false, ws_s, ws_g, ws, &pt);
                     n_runs_max = max(n_runs_max, R);
                     broot = ccl_largest(cta, g, ws, R, area, sx, sy);
                 }
@@ -444,17 +459,17 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
                 cta_sync();
                 pt.tick();   // 7 centroid labelling
                 // ---- P7: exclusions ------------------------------------------------
-                if (a.n_excl > 0) { apply_exclusions(MA, g, a.excl, a.n_excl, dx, dy); cta_sync(); }
+                if (a.n_excl > 0) { apply_exclusions(S, g, a.excl, a.n_excl, dx, dy); cta_sync(); }
             }
             // ---- P8: seg mask out -------------------------------------------------
-            if (mode == MODE_FULL && rs.solid && a.n_excl == 0) seg_area = rs.area;      // one solid blob, untouched since the row scan: its area is the mask's
-            else seg_area = cta_popcount(cta, MA, g);
-            if (cfg_seg_stats) mask_sums(cta, MA, g, cfg_seg_stats + (long long)uid * 3);     // CSV export's mask_stats, optional
-            if (seg_out) store_mask_bytes(MA, g, seg_out);
-            if (cfg_seg_bits) store_mask_words(MA, g, bits_at(cfg_seg_bits));
+            if (rs.solid && a.n_excl == 0) seg_area = rs.area;      // one solid blob, untouched since the row scan: its area is the mask's
+            else seg_area = cta_popcount(cta, S, g);
+            if (cfg_seg_stats) mask_sums(cta, S, g, cfg_seg_stats + (long long)uid * 3);     // CSV export's mask_stats, optional
+            if (seg_out) store_mask_bytes(S, g, seg_out);
+            if (cfg_seg_bits) store_mask_words(S, g, bits_at(cfg_seg_bits));
             pt.tick();   // 8 exclusions + seg mask out
             if (mode == MODE_SEG_ONLY) {
-                write_record(a, uid, img, unit, otsu_t, seg_area, 0, 0, 0, 0, 0, 0, cx, cy, 0, n_runs_max);
+                write_record(a, uid, img, unit, otsu_t, seg_area, 0, 0, 0, VI_STATUS_SEGMENTED, dx, dy, cx, cy, 0, n_runs_max);
                 return;
             }
         }
@@ -636,8 +651,8 @@ __device__ __forceinline__ void process_unit(const KArgs& a, int uid, unsigned c
     pt.tick();   // 15 defect mask out + record
 }
 
-template <bool PROF, bool SPEC, bool GMEM>
-__global__ void __launch_bounds__(kThreads, 1) vi_unit_kernel(const __grid_constant__ KArgs a) {
+template <bool PROF, bool SPEC, bool GMEM, bool SEG>
+__device__ __forceinline__ void unit_kernel_body(const KArgs& a) {
     extern __shared__ __align__(128) unsigned char smem_raw[];      // (128: destination alignment of the tensor copies)
     __shared__ UnitShared sh_raw;
     // The two shared-memory bases are made opaque once: ptxas otherwise re-derives them (S2UR SR_CgaCtaId + a chain
@@ -659,9 +674,20 @@ __global__ void __launch_bounds__(kThreads, 1) vi_unit_kernel(const __grid_const
     if (SPEC && a.tma_ok && (int)blockIdx.x < n_total)           // the first unit's crop arrives the same way as the later ones
         cta.gpending = gather_issue_tma(a, blockIdx.x, smem, a.layout.stage_bytes, &sh.gather_mbar) ? 1 : 0;
     for (int uid = blockIdx.x; uid < n_total; uid += gridDim.x) {
-        process_unit<PROF, SPEC, GMEM>(a, uid, base, smem, sh, cta);
+        process_unit<PROF, SPEC, GMEM, SEG>(a, uid, base, smem, sh, cta);
         cta_sync();
     }
+}
+
+template <bool PROF, bool SPEC, bool GMEM>
+__global__ void __launch_bounds__(kThreads, 1) vi_unit_kernel(const __grid_constant__ KArgs a) {
+    unit_kernel_body<PROF, SPEC, GMEM, false>(a);
+}
+
+// The default configuration in the segmentation-only mode (process_unit: SPEC && SEG).
+template <bool PROF>
+__global__ void __launch_bounds__(kThreads, 1) vi_seg_kernel(const __grid_constant__ KArgs a) {
+    unit_kernel_body<PROF, true, false, true>(a);
 }
 
 }  // namespace vi

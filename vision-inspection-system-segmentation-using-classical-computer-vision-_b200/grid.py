@@ -95,6 +95,22 @@ def grid_to_json(grid: Grid) -> dict:
     }
 
 
+def ref_centroids_from_records(records, image=0) -> Dict[int, Tuple[float, float]]:
+    """{unit: (cx, cy)} of one image's records (RECORD_DTYPE, [n, units] or [n * units] with the image field): the
+    pre-exclusion centroids run_segmentation_all stores from the reference image (indexing_ui.py:2283-2289).  Units
+    without a segmented component (NaN) are left out, as the reference leaves them out.  Assign the result to
+    `Grid.ref_centroids`; `save_grid` writes it as exclusion_alignment.ref_centroids."""
+    import numpy as np
+    r = np.asarray(records).reshape(-1)
+    r = r[r['image'] == int(image)]
+    out = {}
+    for rec in r:
+        cx, cy = float(rec['cx']), float(rec['cy'])
+        if cx == cx and cy == cy:
+            out[int(rec['unit'])] = (cx, cy)
+    return out
+
+
 def save_grid(path, grid: Grid):
     with open(path, "w") as f:
         json.dump(grid_to_json(grid), f, indent=2)

@@ -4,7 +4,7 @@ same error behaviour) running on the B200 through the C ABI.
 ``import segmentation`` in the reference UI keeps working when this module is put
 in its place (INTEGRATION.md).  New in the same style: ``detect_defects`` (the
 compute body of ``MainWindow._detect_defects_on_pix``, indexing_ui.py:1471-1572,
-minus Qt) and ``inspect_batch``.  No CPU fallback: without a CUDA device or the
+minus Qt), ``inspect_batch`` and ``segment_batch``.  No CPU fallback: without a CUDA device or the
 built extension every compute call raises."""
 from __future__ import annotations
 
@@ -91,3 +91,15 @@ def inspect_batch(frames, grid, params=None, is_reference=False):
     return (rec.reshape(n, insp.n_units),
             [insp.split_masks(seg, i) for i in range(n)],
             [insp.split_masks(dfm, i) for i in range(n)])
+
+
+def segment_batch(frames, grid, params=None, is_reference=False):
+    """run_segmentation_all (indexing_ui.py:2203-2368) for every unit of every frame, without the defect detector.
+    frames: uint8 [n, H, W] host array; grid: a vi_b200.grid.Grid.  Returns (records, seg_masks): records [n, units]
+    (status STATUS_SEGMENTED; cx / cy feed `grid.ref_centroids_from_records`), masks as per-image lists of (h, w)
+    arrays."""
+    insp = default_inspector()
+    insp.configure(grid, is_reference=is_reference)
+    rec, seg = insp.segment_batch_host(np.asarray(frames), params)
+    n = len(frames)
+    return rec.reshape(n, insp.n_units), [insp.split_masks(seg, i) for i in range(n)]
